@@ -2,7 +2,7 @@
 """Headline benchmark: TPS_PP rectifier forward (BASELINE.json configs[1]) -- img/s and the fused
 warp kernel's HBM roofline fraction.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step = one ``TPS_PP.forward`` over a batch of 256 synthetic feature maps per GPU
 (x [256,64,16,64], outs 2x[256,32,32,128], fp32, F=32 -- the only geometry the reference module
@@ -33,6 +33,21 @@ TF32X3_CEILING = 1125.0 / 3.0      # TFLOP/s: nominal dense tf32 rate, three MMA
 STAGE_GFLOP_PER_IMG = 0.607        # stem 7.1 M + layer1 251.7 M + layer2 348.2 M (resnet_v2_large.py:109-135; 2 FLOP per MAC)
 HEAD_GFLOP_PER_IMG = 0.82          # SURVEY 8(d): convs 720.6 M + DGAB/MLP 76.4 M + score 21.4 M + localization 1.1 M
 WARP_CONST_BYTES = 131072 + 4900 + 8192
+DUMP_LIMIT_BYTES = 60 * 10 ** 6        # array data of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def _dump_outputs(path, arrays):
+    """Write what a caller of the timed path received in its last step to path/<name>.npy as float32.  The arrays share
+    their leading (batch) dimension; when together they exceed DUMP_LIMIT_BYTES, the same fixed, seeded sample of batch
+    indices is kept from each, so two builds run with the same arguments write the same elements."""
+    batch = next(iter(arrays.values())).shape[0]
+    per_item = sum(t[0].numel() * 4 for t in arrays.values())
+    keep = min(batch, DUMP_LIMIT_BYTES // per_item)
+    idx = torch.from_numpy(np.sort(np.random.RandomState(0).choice(batch, keep, replace=False)))
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t[idx.to(t.device)].float().cpu().numpy())
+    print(f"bench: wrote {', '.join(sorted(arrays))} of {keep} of {batch} items to {path}", file=sys.stderr, flush=True)
 
 
 def _warp_traffic():
@@ -345,7 +360,7 @@ def run_ours(args):
         barrier()
         e0.record()
         for _ in range(args.steps):
-            m(x, [o0, o1])
+            r = m(x, [o0, o1])
             launches += N.last_launch_count() + m._last_head_launches
         e1.record()
         barrier()
@@ -353,6 +368,9 @@ def run_ours(args):
         total_ms = e0.elapsed_time(e1)
         warp_ms = [a.elapsed_time(b) for a, b in m.warp_events]
         m.warp_events = None
+        if args.dump_outputs and rank == 0:
+            _dump_outputs(args.dump_outputs, {k: v for k, v in r.items() if v is not None})
+        del r
 
         # per-launch times of the head (CUDA events recorded by the library around each of its kernels), taken in a
         # separate short pass after the timed region so the event records cannot perturb `value`
@@ -752,12 +770,15 @@ def run_classical(args):
         barrier()
         e0.record()
         for _ in range(args.steps):
-            step(img)
+            out = step(img)
             launches += N.last_launch_count()
         e1.record()
         barrier()
         clocks = sampler.stop()
         total_ms = e0.elapsed_time(e1)
+        if args.dump_outputs and rank == 0:
+            _dump_outputs(args.dump_outputs, {"output": out})
+        del out
         # end to end with host buffers: H2D of the images + control points, D2H of the rectified images, every step
         himg, hcp = img.cpu().pin_memory(), cp.cpu().pin_memory()
         hout = torch.empty_like(himg).pin_memory()
@@ -882,7 +903,14 @@ def main():
                     help="head arithmetic: tcgen05 split-fp32 (default, fp32-level accuracy; tc3x = all-tf32 3xTF32 convs), CUDA-core fp32, "
                          "tcgen05 with bf16 conv operands (reduced precision, reported separately), or "
                          "cuDNN/cuBLAS library ops")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (rank 0's shard) to DIR/<name>.npy as float32; "
+                         "above 64 MB in all, the same seeded sample of images is kept from every array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.workload == "classical64x256":
         if args.batch == BATCH_PER_GPU:
             args.batch = 1024

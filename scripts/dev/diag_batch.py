@@ -1,5 +1,5 @@
-import sys, torch, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, torch, numpy as np
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', '..'))
 from oracle import tpspp_oracle as O
 import tps_pp_b200 as T
 DEV='cuda:0'

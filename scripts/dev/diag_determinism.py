@@ -1,6 +1,6 @@
 """Dev tool: run the native head twice on the same inputs and report which workspace intermediates differ."""
-import sys, torch, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, torch, numpy as np
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', '..'))
 from oracle import tpspp_oracle as O
 import tps_pp_b200 as T
 from tps_pp_b200 import _native as N, functional as TF

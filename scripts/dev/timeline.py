@@ -1,8 +1,8 @@
 """Dev tool: prints the clock64 timeline written by an INSTRUMENTED build of libtpspp.so (a temporary g_tl device array +
 tpspp_dbg_read export patched into conv_tma_kernel by hand; see profiles/r02_conv_experiments.md).  The last conv_tma launch
 of the forward (dec3: 18 chunks per tile) is what remains in the buffer.  It does not work against the shipped library."""
-import sys, ctypes, torch, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, ctypes, torch, numpy as np
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', '..'))
 import tps_pp_b200 as T
 from tps_pp_b200 import _native as N
 DEV = 'cuda:0'
