@@ -371,6 +371,23 @@ TPSPP_API int tpspp_attn_decode(const tpspp_attn_cfg* cfg, const float* q, float
                                 const int32_t* kv_lens /* [batch] device pointer or NULL */, const float* k_new, const float* v_new,
                                 float* out, tpspp_stream_t stream);
 
+/* ---- Multi-head self-attention over whole sequences: the attention of NRTREncoder (reference encoders/nrtr_encoder.py:66-87;
+ * TFEncoderLayer -> MultiHeadAttention / ScaledDotProductAttention, common/modules/transformer_module.py:24-34,74-98) with the
+ * encoder's source mask (_get_mask); the reference-side binding is tps_pp_b200/nrtr.py::NRTREncoder.
+ *   out[b,i,h,:] = sum_{j < len(b)} softmax_j((q[b,i,h,:] / temperature) . K[b,j,h,:]) V[b,j,h,:]   for every i < seq_len
+ * q / k / v: token-major [batch*seq_len, heads*64] fp32 rows `row_stride` floats apart (column slices of one fused q|k|v
+ * projection allowed); out: [batch*seq_len, heads*64] row-major.  len(b) = kv_lens[b] (clamped to [0, seq_len]) or seq_len.
+ * Every query row is computed, also i >= len(b); len(b) = 0 gives NaN rows (the reference's soft-max over no key).
+ * fp32 on CUDA cores, online soft-max; any seq_len >= 1.  Pointers 16-byte aligned. */
+typedef struct tpspp_attn_encode_cfg {
+  int32_t batch, heads, head_dim;   /* batch <= 65535; head_dim = 64                                        */
+  int32_t seq_len;                  /* T: tokens per image (queries and keys)                               */
+  float temperature;                /* d_k ** 0.5 in the reference                                          */
+  int32_t row_stride;               /* floats between consecutive token rows of q / k / v (0 = heads*64; a multiple of 4) */
+} tpspp_attn_encode_cfg;
+TPSPP_API int tpspp_attn_encode(const tpspp_attn_encode_cfg* cfg, const float* q, const float* k, const float* v,
+                                const int32_t* kv_lens /* [batch] device pointer or NULL */, float* out, tpspp_stream_t stream);
+
 /* Number of kernel launches the most recent call on this host thread enqueued
  * (bench.py uses it to report gpu_launches). */
 TPSPP_API int tpspp_last_launch_count(void);

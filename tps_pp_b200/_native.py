@@ -63,6 +63,12 @@ class AttnCfg(Structure):
                 ("temperature", c_float), ("q_stride", c_int32), ("new_stride", c_int32), ("kv_head_major", c_int32)]
 
 
+class AttnEncodeCfg(Structure):
+    """Mirror of ``tpspp_attn_encode_cfg`` (include/tpspp.h)."""
+    _fields_ = [("batch", c_int32), ("heads", c_int32), ("head_dim", c_int32), ("seq_len", c_int32), ("temperature", c_float),
+                ("row_stride", c_int32)]
+
+
 class LinearCfg(Structure):
     """Mirror of ``tpspp_linear_cfg`` (include/tpspp.h)."""
     _fields_ = [("rows", ctypes.c_int64), ("in_features", c_int32), ("out_features", c_int32), ("weight_batches", c_int32),
@@ -106,6 +112,7 @@ _SIGNATURES = {
     "tpspp_locnet_workspace_bytes": (c_size_t, [POINTER(LocnetCfg)]),
     "tpspp_locnet_fwd": (c_int, [POINTER(LocnetCfg), c_void_p, POINTER(c_void_p), c_void_p, c_void_p, c_void_p]),
     "tpspp_attn_decode": (c_int, [POINTER(AttnCfg)] + [c_void_p] * 8),
+    "tpspp_attn_encode": (c_int, [POINTER(AttnEncodeCfg)] + [c_void_p] * 6),
     "tpspp_linear_fwd_ex": (c_int, [POINTER(LinearCfg)] + [c_void_p] * 4 + [c_int32] + [c_void_p] * 3),
     "tpspp_linear_ln_fwd": (c_int, [POINTER(LinearCfg)] + [c_void_p] * 4 + [c_int32] + [c_void_p] * 3 + [ctypes.c_float] + [c_void_p] * 3),
     "tpspp_linear_workspace_bytes": (c_size_t, [POINTER(LinearCfg)]),

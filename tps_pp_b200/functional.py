@@ -630,3 +630,37 @@ def attn_decode(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, k
         N.check(N.lib().tpspp_attn_decode(ctypes.byref(cfg), _ptr(q), _ptr(k), _ptr(v), _ptr(kv_lens), _ptr(k_new), _ptr(v_new),
                                           _ptr(out), _stream(q)), "tpspp_attn_decode")
     return out
+
+
+def attn_encode(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, seq_len: int, temperature: float,
+                kv_lens: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Multi-head self-attention over whole sequences (``tpspp_attn_encode``): q / k / v token-major [B*T, heads*64] -> out
+    [B*T, heads*64]; image b's queries (all T of them) attend to its keys ``j < kv_lens[b]`` (int32 on the device) or to all T.
+    ``q`` / ``k`` / ``v`` may be column slices of one fused projection: unit stride along the features, one common row stride.
+    ``out`` (optional) must be a contiguous fp32 tensor of that shape on the same device.  Forward only."""
+    for nm, t in (("q", q), ("k", k), ("v", v)):
+        _require_cuda(nm, t, torch.float32)
+    rows, d = q.shape if q.dim() == 2 else (-1, -1)
+    seq_len = int(seq_len)
+    if seq_len < 1 or d != heads * 64 or rows % seq_len:
+        raise RuntimeError(f"tps_pp_b200: attn_encode q must be [B*T, heads*64] with T = {seq_len} >= 1, got {tuple(q.shape)} "
+                           f"for {heads} heads")
+    b = rows // seq_len
+    for nm, t in (("q", q), ("k", k), ("v", v)):
+        if t.shape != (rows, d) or t.stride(1) != 1 or t.device != q.device:
+            raise RuntimeError(f"tps_pp_b200: attn_encode `{nm}` must be [{rows}, {d}] on {q.device} with unit stride along the features")
+    stride = int(q.stride(0)) if rows > 1 else d
+    if rows > 1 and (k.stride(0) != stride or v.stride(0) != stride):
+        raise RuntimeError("tps_pp_b200: attn_encode q / k / v must share one row stride")
+    if kv_lens is not None and (kv_lens.dtype != torch.int32 or not kv_lens.is_cuda or kv_lens.numel() != b
+                                or kv_lens.device != q.device or not kv_lens.is_contiguous()):
+        raise RuntimeError("tps_pp_b200: kv_lens must be a contiguous int32 tensor on the device of q with one entry per image")
+    if out is None:
+        out = torch.empty((rows, d), dtype=torch.float32, device=q.device)
+    elif (out.dtype != torch.float32 or out.device != q.device or tuple(out.shape) != (rows, d) or not out.is_contiguous()):
+        raise RuntimeError(f"tps_pp_b200: attn_encode `out` must be a contiguous fp32 [{rows}, {d}] tensor on {q.device}")
+    cfg = N.AttnEncodeCfg(b, heads, 64, seq_len, float(temperature), stride)
+    with torch.cuda.device(q.device):
+        N.check(N.lib().tpspp_attn_encode(ctypes.byref(cfg), _ptr(q), _ptr(k), _ptr(v), _ptr(kv_lens), _ptr(out), _stream(q)),
+                "tpspp_attn_encode")
+    return out

@@ -1,6 +1,9 @@
-"""Drop-in ``NRTRDecoder`` (registry ``DECODERS``; reference mmocr/models/textrecog/decoders/nrtr_decoder.py:13-177 over
+"""Drop-in ``NRTRDecoder`` (registry ``DECODERS``) and ``NRTREncoder`` (registry ``ENCODERS``, at the end of this file;
+the encoder's attention is ``tpspp_attn_encode``).
+
+``NRTRDecoder``: reference mmocr/models/textrecog/decoders/nrtr_decoder.py:13-177 over
 ``TFDecoderLayer`` / ``MultiHeadAttention`` / ``PositionwiseFeedForward`` / ``PositionalEncoding``,
-common/layers/transformer_layers.py:76-167, common/modules/transformer_module.py:36-175) -- SURVEY.md section 8f rank 2.
+common/layers/transformer_layers.py:76-167, common/modules/transformer_module.py:36-175 -- SURVEY.md section 8f rank 2.
 
 Same constructor kwargs, sub-module names and ``state_dict`` keys (``trg_word_emb``, ``position_enc.position_table``,
 ``layer_stack.{i}.{norm1,norm2,norm3,self_attn.{linear_q,linear_k,linear_v,fc},enc_attn.{...},mlp.{w_1,w_2}}``,
@@ -27,7 +30,30 @@ import torch.nn.functional as F
 
 from . import functional as TF
 from .rectifier import _BaseModule
-from .registry import DECODERS
+from .registry import DECODERS, ENCODERS
+
+
+def valid_lengths(t: int, img_metas) -> Optional[list]:
+    """Valid length of each image's ``t``-token source sequence, ``min(t, ceil(t * valid_ratio))`` -- the source mask of both
+    ``NRTRDecoder._get_mask`` (nrtr_decoder.py:114-127) and ``NRTREncoder._get_mask`` (nrtr_encoder.py); None without metas."""
+    if img_metas is None:
+        return None
+    return [min(t, math.ceil(t * meta.get("valid_ratio", 1.0))) for meta in img_metas]
+
+
+def _attn_lib(att, n_head, d_k, q, k, v, mask):
+    """``MultiHeadAttention.forward`` (transformer_module.py:24-34,74-98) on torch ops, eval mode; ``mask`` [N, Lk] or
+    [N, Lq, Lk], 0 = masked key."""
+    b, lq, _ = q.shape
+    lk = k.shape[1]
+    qq = att.linear_q(q).view(b, lq, n_head, d_k).transpose(1, 2)
+    kk = att.linear_k(k).view(b, lk, n_head, d_k).transpose(1, 2)
+    vv = att.linear_v(v).view(b, lk, n_head, -1).transpose(1, 2)
+    a = torch.matmul(qq / d_k ** 0.5, kk.transpose(2, 3))
+    if mask is not None:
+        a = a.masked_fill((mask.unsqueeze(1) if mask.dim() == 3 else mask[:, None, None, :]) == 0, float("-inf"))
+    out = torch.matmul(F.softmax(a, dim=-1), vv).transpose(1, 2).contiguous().view(b, lq, -1)
+    return att.fc(out)
 
 
 def _sinusoid_table(n_position: int, d_hid: int) -> torch.Tensor:
@@ -81,17 +107,7 @@ class NRTRDecoder(_BaseModule):
 
     # ------------------------------------------------------------------ reference algorithm on torch ops
     def _attn_lib(self, att, q, k, v, mask):
-        b, lq, _ = q.shape
-        lk = k.shape[1]
-        h, dk = self.n_head, self.d_k
-        qq = att.linear_q(q).view(b, lq, h, dk).transpose(1, 2)
-        kk = att.linear_k(k).view(b, lk, h, dk).transpose(1, 2)
-        vv = att.linear_v(v).view(b, lk, h, dk).transpose(1, 2)
-        a = torch.matmul(qq / dk ** 0.5, kk.transpose(2, 3))
-        if mask is not None:
-            a = a.masked_fill((mask.unsqueeze(1) if mask.dim() == 3 else mask[:, None, None, :]) == 0, float("-inf"))
-        out = torch.matmul(F.softmax(a, dim=-1), vv).transpose(1, 2).contiguous().view(b, lq, h * dk)
-        return att.fc(out)
+        return _attn_lib(att, self.n_head, self.d_k, q, k, v, mask)
 
     def _attention(self, trg_seq, src, src_mask=None):
         """nrtr_decoder.py:93-112 (pre-norm layers, transformer_layers.py:152-165); dropout is the identity in eval mode."""
@@ -114,8 +130,8 @@ class NRTRDecoder(_BaseModule):
             return None
         n, t, _ = logit.size()
         mask = logit.new_zeros((n, t))
-        for i, meta in enumerate(img_metas):
-            mask[i, :min(t, math.ceil(t * meta.get("valid_ratio", 1.0)))] = 1
+        for i, width in enumerate(valid_lengths(t, img_metas)):
+            mask[i, :width] = 1
         return mask
 
     def forward_train(self, feat, out_enc, targets_dict, img_metas):
@@ -148,8 +164,7 @@ class NRTRDecoder(_BaseModule):
         n, t_src, d = out_enc.shape
         lens = None
         if img_metas is not None:
-            lens = torch.tensor([min(t_src, math.ceil(t_src * m.get("valid_ratio", 1.0))) for m in img_metas], dtype=torch.int32,
-                                device=out_enc.device)
+            lens = torch.tensor(valid_lengths(t_src, img_metas), dtype=torch.int32, device=out_enc.device)
         if not getattr(self, "decode_graph", True) or torch.cuda.is_current_stream_capturing():
             return self._decode(out_enc, lens)
         key = (n, t_src, out_enc.device.index, lens is not None, tuple((p.data_ptr(), p._version) for p in self.parameters()))
@@ -246,3 +261,111 @@ class NRTRDecoder(_BaseModule):
         if train_mode:
             return self.forward_train(feat, out_enc, targets_dict, img_metas)
         return self.forward_test(feat, out_enc, img_metas)
+
+
+_PRE_NORM = ("norm", "self_attn", "norm", "ffn")
+
+
+@ENCODERS.register_module()
+class NRTREncoder(_BaseModule):
+    """Drop-in ``NRTREncoder`` (registry ``ENCODERS``; reference mmocr/models/textrecog/encoders/nrtr_encoder.py over pre-norm
+    ``TFEncoderLayer`` / ``MultiHeadAttention`` / ``PositionwiseFeedForward``, common/layers/transformer_layers.py,
+    common/modules/transformer_module.py).  Same constructor kwargs, ``state_dict`` keys (``layer_stack.{i}.{attn.{linear_q,
+    linear_k,linear_v,fc},norm1,mlp.{w_1,w_2},norm2}``, ``layer_norm``) and creation order as the reference.
+
+    ``forward(feat [N, C, H, W], img_metas) -> [N, H*W, C]``.  In eval mode under ``torch.no_grad()`` on fp32 CUDA tensors it
+    runs natively: per layer one fused q|k|v dense layer, ``tpspp_attn_encode`` over the whole sequence with the valid-ratio
+    key mask, ``fc`` with the residual add and ``norm2`` in its epilogue, ``w_1`` with GELU, ``w_2`` with the residual add and
+    the next layer's ``norm1`` (after the last layer: the final ``layer_norm``) -- the tcgen05 3xTF32 dense kernels of
+    ``NRTRDecoder``.  ``forward_library`` is the reference algorithm on torch ops; ``forward`` uses it while autograd records,
+    in training mode, for head sizes other than 64 or model widths that are not a multiple of 128, and for an image whose
+    valid length is 0 (the reference's soft-max over no key: NaN rows).  Dropout is the identity in eval mode and is not
+    applied by either path (training runs in mmocr)."""
+
+    def __init__(self, n_layers=6, n_head=8, d_k=64, d_v=64, d_model=512, d_inner=256, dropout=0.1, init_cfg=None, **kwargs):
+        super().__init__(init_cfg=init_cfg)
+        qkv_bias = kwargs.pop("qkv_bias", False)
+        order = kwargs.pop("operation_order", None)
+        act_cfg = kwargs.pop("act_cfg", None)
+        if kwargs:
+            raise TypeError(f"tps_pp_b200.NRTREncoder got unexpected keyword arguments {sorted(kwargs)}")
+        if order is not None and tuple(order) != _PRE_NORM:
+            raise ValueError(f"tps_pp_b200.NRTREncoder implements the pre-norm layer {_PRE_NORM} only, got operation_order={order!r}")
+        if act_cfg is not None and dict(act_cfg) not in (dict(type="mmcv.GELU"), dict(type="GELU")):
+            raise ValueError(f"tps_pp_b200.NRTREncoder implements the GELU feed-forward only, got act_cfg={act_cfg!r}")
+        self.n_layers, self.n_head, self.d_k, self.d_v, self.d_model = n_layers, n_head, d_k, d_v, d_model
+        layers = []
+        for _ in range(n_layers):
+            lyr = nn.Module()
+            lyr.attn = _mha(n_head, d_model, d_k, d_v, qkv_bias)
+            lyr.norm1 = nn.LayerNorm(d_model)
+            mlp = nn.Module()
+            mlp.w_1 = nn.Linear(d_model, d_inner)
+            mlp.w_2 = nn.Linear(d_inner, d_model)
+            lyr.mlp = mlp
+            lyr.norm2 = nn.LayerNorm(d_model)
+            layers.append(lyr)
+        self.layer_stack = nn.ModuleList(layers)
+        self.layer_norm = nn.LayerNorm(d_model)
+        self.last_forward_native = None
+
+    def _native_ok(self, feat, lens) -> bool:
+        return (not self.training and not torch.is_grad_enabled() and feat.dtype == torch.float32 and feat.dim() == 4
+                and self.d_k == 64 and self.d_v == 64 and self.d_model == self.n_head * 64 and self.d_model % 128 == 0
+                and self.d_model <= 1024 and feat.shape[1] == self.d_model and (lens is None or min(lens, default=1) > 0))
+
+    def forward(self, feat, img_metas=None):
+        """nrtr_encoder.py:66-87: [N, C, H, W] -> [N, H*W, C]."""
+        if not feat.is_cuda:
+            raise RuntimeError("tps_pp_b200.NRTREncoder runs on CUDA (sm_100a) tensors only; there is no CPU fallback "
+                               "(forward_library is the torch-ops A/B path)")
+        lens = valid_lengths(feat.shape[2] * feat.shape[3], img_metas)
+        self.last_forward_native = self._native_ok(feat, lens)
+        if self.last_forward_native:
+            return self._encode(feat, lens)
+        return self.forward_library(feat, img_metas)
+
+    def forward_library(self, feat, img_metas=None):
+        """The reference's algorithm on torch ops (any device): pre-norm layers x += attn(norm1(x)); x += w_2(GELU(w_1(norm2(x))))."""
+        n, c, h, w = feat.size()
+        x = feat.view(n, c, h * w).permute(0, 2, 1).contiguous()
+        lens = valid_lengths(h * w, img_metas)
+        mask = None
+        if lens is not None:
+            mask = x.new_zeros((n, h * w))
+            for i, width in enumerate(lens):
+                mask[i, :width] = 1
+        for lyr in self.layer_stack:
+            hn = lyr.norm1(x)
+            x = x + _attn_lib(lyr.attn, self.n_head, self.d_k, hn, hn, hn, mask)
+            x = x + lyr.mlp.w_2(F.gelu(lyr.mlp.w_1(lyr.norm2(x))))
+        return self.layer_norm(x)
+
+    @torch.no_grad()
+    def _encode(self, feat, lens):
+        n, c, h, w = feat.shape
+        t = h * w
+        dev = feat.device
+        rows = (n * t + 127) // 128 * 128              # the tensor-core dense kernels take multiples of 128 rows
+        x = torch.zeros((rows, c), dtype=torch.float32, device=dev)
+        x[: n * t].view(n, t, c).copy_(feat.reshape(n, c, t).permute(0, 2, 1))
+        att = torch.zeros((rows, c), dtype=torch.float32, device=dev)
+        kv_lens = torch.tensor(lens, dtype=torch.int32, device=dev) if lens is not None else None
+        layers = list(self.layer_stack)
+        hn = (layers[0].norm1 if layers else self.layer_norm)(x).contiguous()    # LN(x) for the next sub-layer
+        temp = self.d_k ** 0.5
+        for li, lyr in enumerate(layers):
+            a, mlp = lyr.attn, lyr.mlp
+            # the operand images of the layer's dense weights are laid out once per call (each is used once)
+            qkv = TF.PreparedLinear(torch.cat([a.linear_q.weight, a.linear_k.weight, a.linear_v.weight], 0),
+                                    None if a.linear_q.bias is None else torch.cat([a.linear_q.bias, a.linear_k.bias, a.linear_v.bias], 0),
+                                    rows)(hn)
+            # q, k, v are column slices of the fused projection
+            TF.attn_encode(qkv[: n * t, :c], qkv[: n * t, c:2 * c], qkv[: n * t, 2 * c:], self.n_head, t, temp, kv_lens=kv_lens,
+                           out=att[: n * t])
+            # x += fc(att) and hn = norm2(x): residual and the next LayerNorm in the kernel that finishes the dense layer
+            TF.PreparedLinear(a.fc.weight, a.fc.bias, rows)(att, out=x, residual=x, ln=lyr.norm2, ln_out=hn)
+            mid = TF.PreparedLinear(mlp.w_1.weight, mlp.w_1.bias, rows)(hn, gelu=True)
+            nxt = layers[li + 1].norm1 if li + 1 < len(layers) else self.layer_norm
+            TF.PreparedLinear(mlp.w_2.weight, mlp.w_2.bias, rows)(mid, out=x, residual=x, ln=nxt, ln_out=hn)   # x += w_2(GELU(w_1(LN(x))))
+        return hn[: n * t].view(n, t, c)

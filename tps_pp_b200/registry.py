@@ -44,6 +44,9 @@ class Registry:
 BACKBONES = Registry("backbone")
 PREPROCESSOR = Registry("preprocessor")
 DECODERS = Registry("decoder")
+ENCODERS = Registry("encoder")
+CONVERTORS = Registry("convertor")
+RECOGNIZERS = Registry("recognizer")
 
 
 def build_backbone(cfg):
@@ -62,13 +65,35 @@ def build_decoder(cfg):
     return DECODERS.build(cfg)
 
 
+def build_encoder(cfg):
+    """reference mmocr/models/builder.py (``ENCODERS``); used for ``encoder`` at recognizer/encode_decode_recognizer.py."""
+    return ENCODERS.build(cfg)
+
+
+def build_convertor(cfg):
+    """reference mmocr/models/builder.py (``CONVERTORS``); used for ``label_convertor`` at recognizer/encode_decode_recognizer.py."""
+    return CONVERTORS.build(cfg)
+
+
+def build_recognizer(cfg):
+    """``dict(type='NRTR', backbone=..., tpsnet=..., encoder=..., decoder=..., label_convertor=...)`` -> the recogniser."""
+    return RECOGNIZERS.build(cfg)
+
+
 def register_into_mmocr(force: bool = True) -> bool:
-    """Register the B200 modules into a real MMOCR install, replacing the stock classes."""
+    """Register the B200 modules into a real MMOCR install, replacing the stock classes (``ENCODERS`` too where the install
+    exposes that registry)."""
     try:
         from mmocr.models.builder import BACKBONES as MB, DECODERS as MD, PREPROCESSOR as MP  # type: ignore
     except Exception:
         return False
-    for reg, ours in ((MB, BACKBONES), (MP, PREPROCESSOR), (MD, DECODERS)):
+    pairs = [(MB, BACKBONES), (MP, PREPROCESSOR), (MD, DECODERS)]
+    try:
+        from mmocr.models.builder import ENCODERS as ME  # type: ignore
+        pairs.append((ME, ENCODERS))
+    except Exception:
+        pass
+    for reg, ours in pairs:
         for key, cls in ours.module_dict.items():
             reg.register_module(name=key, force=force, module=cls)
     return True
