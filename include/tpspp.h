@@ -388,6 +388,27 @@ typedef struct tpspp_attn_encode_cfg {
 TPSPP_API int tpspp_attn_encode(const tpspp_attn_encode_cfg* cfg, const float* q, const float* k, const float* v,
                                 const int32_t* kv_lens /* [batch] device pointer or NULL */, float* out, tpspp_stream_t stream);
 
+/* ---- Text-recognition test pipeline: mmocr 0.4 ResizeOCR -> ToTensorOCR -> NormalizeOCR (reference
+ * datasets/pipelines/ocr_transforms.py:67-130) for a whole ragged batch of uint8 images in one launch.
+ *   packed  uint8 HWC images, 3 channels in the caller's channel order (no BGR/RGB swap), one after the other
+ *   desc    [n][4] int64 device array: byte offset of the image in `packed`, h, w, resize_w (the width ResizeOCR chose)
+ *   out     [n, 3, out_h, out_w] fp32 NCHW
+ * Pixel (c, y, x) of image i: x < resize_w: cv2.resize(img, (resize_w, out_h), INTER_LINEAR) on uint8 (OpenCV's fixed-point
+ * arithmetic, bit for bit); x >= resize_w: pad_value (mmcv.impad).  Then ((float)u8 / 255 - mean[c]) / std[c] in fp32 with
+ * IEEE divisions (torchvision to_tensor + normalize).  The library cannot read the descriptors without a host sync, so it does
+ * not validate them; every read of `packed` is bounded by packed_bytes, so a corrupt descriptor gives wrong pixels but never an
+ * out-of-range access.  The Python wrapper (tps_pp_b200/functional.py::ocr_prep) checks descriptors on the host. */
+typedef struct tpspp_ocr_prep_cfg {
+  int32_t n;                /* images                                                               */
+  int32_t out_h, out_w;     /* ResizeOCR height, max_width                                          */
+  float mean[3], std[3];    /* NormalizeOCR, per channel of the caller's order; std != 0            */
+  int32_t pad_value;        /* ResizeOCR img_pad_value, uint8 domain [0, 255]                       */
+  int32_t flags;            /* 0 (reserved)                                                         */
+  int64_t packed_bytes;     /* size of `packed`: every read stays below it                          */
+} tpspp_ocr_prep_cfg;
+TPSPP_API int tpspp_ocr_prep(const tpspp_ocr_prep_cfg* cfg, const uint8_t* packed, const int64_t* desc, float* out,
+                             tpspp_stream_t stream);
+
 /* Number of kernel launches the most recent call on this host thread enqueued
  * (bench.py uses it to report gpu_launches). */
 TPSPP_API int tpspp_last_launch_count(void);

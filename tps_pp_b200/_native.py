@@ -69,6 +69,12 @@ class AttnEncodeCfg(Structure):
                 ("row_stride", c_int32)]
 
 
+class OcrPrepCfg(Structure):
+    """Mirror of ``tpspp_ocr_prep_cfg`` (include/tpspp.h)."""
+    _fields_ = [("n", c_int32), ("out_h", c_int32), ("out_w", c_int32), ("mean", c_float * 3), ("std", c_float * 3),
+                ("pad_value", c_int32), ("flags", c_int32), ("packed_bytes", ctypes.c_int64)]
+
+
 class LinearCfg(Structure):
     """Mirror of ``tpspp_linear_cfg`` (include/tpspp.h)."""
     _fields_ = [("rows", ctypes.c_int64), ("in_features", c_int32), ("out_features", c_int32), ("weight_batches", c_int32),
@@ -113,6 +119,7 @@ _SIGNATURES = {
     "tpspp_locnet_fwd": (c_int, [POINTER(LocnetCfg), c_void_p, POINTER(c_void_p), c_void_p, c_void_p, c_void_p]),
     "tpspp_attn_decode": (c_int, [POINTER(AttnCfg)] + [c_void_p] * 8),
     "tpspp_attn_encode": (c_int, [POINTER(AttnEncodeCfg)] + [c_void_p] * 6),
+    "tpspp_ocr_prep": (c_int, [POINTER(OcrPrepCfg)] + [c_void_p] * 4),
     "tpspp_linear_fwd_ex": (c_int, [POINTER(LinearCfg)] + [c_void_p] * 4 + [c_int32] + [c_void_p] * 3),
     "tpspp_linear_ln_fwd": (c_int, [POINTER(LinearCfg)] + [c_void_p] * 4 + [c_int32] + [c_void_p] * 3 + [ctypes.c_float] + [c_void_p] * 3),
     "tpspp_linear_workspace_bytes": (c_size_t, [POINTER(LinearCfg)]),

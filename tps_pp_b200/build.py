@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtpspp.so")
 STAMP = os.path.join(HERE, ".libtpspp.stamp")
 SOURCES = ["abi.cu", "warp_fwd.cu", "warp_bwd.cu", "head.cu", "head_tc.cu", "stage.cu", "conv_train.cu", "linear_train.cu", "locnet.cu", "attn_decode.cu",
-           "attn_encode.cu"]
+           "attn_encode.cu", "ocr_prep.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

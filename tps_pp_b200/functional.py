@@ -3,6 +3,7 @@
 ``tps_warp``      fused grid generator + bilinear sampling (reference tps_pp.py:481-496,601-615;
                   tps_preprocessor.py:72-83,270-282)
 ``grid_sample_border`` the sampler alone for an explicit grid (ATen-compatible fp32 coordinates)
+``ocr_prep``      the text-recognition test pipeline (ResizeOCR + ToTensorOCR + NormalizeOCR) for a ragged uint8 batch
 
 Tensors must live on a CUDA device; there is no CPU path.
 """
@@ -11,6 +12,7 @@ from __future__ import annotations
 import ctypes
 from typing import Optional, Tuple
 
+import numpy as np
 import torch
 
 from . import _native as N
@@ -663,4 +665,58 @@ def attn_encode(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, s
     with torch.cuda.device(q.device):
         N.check(N.lib().tpspp_attn_encode(ctypes.byref(cfg), _ptr(q), _ptr(k), _ptr(v), _ptr(kv_lens), _ptr(out), _stream(q)),
                 "tpspp_attn_encode")
+    return out
+
+
+def check_ocr_desc(desc, packed_bytes: int, out_w: int) -> np.ndarray:
+    """Host-side check of the ``tpspp_ocr_prep`` descriptors (the kernel reads them on the device and cannot check them without
+    a host sync): ``desc`` [n, 4] int64 rows (byte offset, h, w, resize_w) of images in a packed uint8 buffer of
+    ``packed_bytes`` bytes.  Raises ``ValueError``; returns the rows as an int64 numpy array."""
+    d = desc.numpy() if isinstance(desc, torch.Tensor) else np.asarray(desc)
+    if isinstance(desc, torch.Tensor) and desc.device.type != "cpu":
+        raise ValueError("tps_pp_b200: ocr_prep descriptors are checked on the host: pass them as a CPU tensor or numpy array")
+    if d.dtype != np.int64 or d.ndim != 2 or d.shape[1] != 4 or d.shape[0] < 1:
+        raise ValueError(f"tps_pp_b200: ocr_prep descriptors must be a non-empty int64 [n, 4] array, got {d.dtype} {d.shape}")
+    off, h, w, rw = d[:, 0], d[:, 1], d[:, 2], d[:, 3]
+    for what, bad in (("h >= 1", h < 1), ("w >= 1", w < 1), ("offset >= 0", off < 0),
+                      (f"1 <= resize_w <= out_w = {out_w}", (rw < 1) | (rw > out_w))):
+        if bad.any():
+            i = int(np.flatnonzero(bad)[0])
+            raise ValueError(f"tps_pp_b200: ocr_prep descriptor {i} {d[i].tolist()} breaks {what}")
+    end = off + h * w * 3
+    past = (end > int(packed_bytes)) | (end < off)
+    if past.any():
+        i = int(np.flatnonzero(past)[0])
+        raise ValueError(f"tps_pp_b200: ocr_prep image {i} {d[i].tolist()} reaches past the end of the {packed_bytes}-byte buffer")
+    return d
+
+
+def ocr_prep(packed: torch.Tensor, desc, out_h: int, out_w: int, mean, std, pad_value: int = 0,
+             out: Optional[torch.Tensor] = None, desc_dev: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """mmocr's ResizeOCR + ToTensorOCR + NormalizeOCR for a ragged batch in one launch (``tpspp_ocr_prep``): ``packed`` uint8
+    HWC 3-channel images one after the other (1-D CUDA tensor), ``desc`` their [n, 4] int64 descriptors (byte offset, h, w,
+    resize_w) ON THE HOST, checked by :func:`check_ocr_desc` before anything is launched -> [n, 3, out_h, out_w] fp32.
+    ``desc_dev``: the same descriptors already on the device (a caller that uploads them with its images in one copy);
+    otherwise they are copied here.  ``out`` (optional) must be a contiguous fp32 tensor of that shape on the same device."""
+    d = check_ocr_desc(desc, packed.numel(), out_w)
+    if len(mean) != 3 or len(std) != 3:
+        raise ValueError(f"tps_pp_b200: ocr_prep takes 3 means and 3 stds, got {len(mean)} and {len(std)}")
+    _require_cuda("packed", packed, torch.uint8)
+    if packed.dim() != 1 or not packed.is_contiguous():
+        raise RuntimeError("tps_pp_b200: ocr_prep `packed` must be a contiguous 1-D uint8 tensor")
+    n = d.shape[0]
+    if desc_dev is None:
+        desc_dev = torch.from_numpy(d).to(packed.device)
+    elif (desc_dev.dtype != torch.int64 or desc_dev.device != packed.device or tuple(desc_dev.shape) != (n, 4)
+          or not desc_dev.is_contiguous()):
+        raise RuntimeError(f"tps_pp_b200: ocr_prep `desc_dev` must be a contiguous int64 [{n}, 4] tensor on {packed.device}")
+    shape = (n, 3, int(out_h), int(out_w))
+    if out is None:
+        out = torch.empty(tuple(max(s, 0) for s in shape), dtype=torch.float32, device=packed.device)
+    elif out.dtype != torch.float32 or out.device != packed.device or tuple(out.shape) != shape or not out.is_contiguous():
+        raise RuntimeError(f"tps_pp_b200: ocr_prep `out` must be a contiguous fp32 {list(shape)} tensor on {packed.device}")
+    cfg = N.OcrPrepCfg(n, int(out_h), int(out_w), (ctypes.c_float * 3)(*[float(m) for m in mean]),
+                       (ctypes.c_float * 3)(*[float(s) for s in std]), int(pad_value), 0, packed.numel())
+    with torch.cuda.device(packed.device):
+        N.check(N.lib().tpspp_ocr_prep(ctypes.byref(cfg), _ptr(packed), _ptr(desc_dev), _ptr(out), _stream(packed)), "tpspp_ocr_prep")
     return out

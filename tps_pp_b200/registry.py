@@ -47,6 +47,8 @@ DECODERS = Registry("decoder")
 ENCODERS = Registry("encoder")
 CONVERTORS = Registry("convertor")
 RECOGNIZERS = Registry("recognizer")
+# the batched GPU test pipeline (tps_pp_b200/pipeline.py); not registered into mmocr: its transforms run per image on the host
+PIPELINES = Registry("pipeline")
 
 
 def build_backbone(cfg):
