@@ -201,7 +201,7 @@ def test_tps_pp_autograd_reaches_every_parameter(native_lib, train_convs, batch)
           f"d batch_img {mx(tx.grad, px.grad) / float(px.grad.abs().max()):.3e}")
     # fp32 head + the TPS solve's 1e2-1e3x rounding amplification (SURVEY F6) + ReLU masks that differ between an fp32 and an
     # fp64 forward at pixels within rounding of zero: percent-level agreement (each convolution alone is checked to 1e-4 in
-    # tests/test_conv_train_gpu.py)
+    # tests/test_conv_train_gpu.py, and at the training batch in tests/test_train_batch_gpu.py)
     assert worst[1] <= 5e-2, worst
     assert mx(tx.grad, px.grad) <= 5e-2 * float(px.grad.abs().max())
 

@@ -287,7 +287,8 @@ __global__ void __launch_bounds__(256) cprime_bwd_kernel(WarpParams p, int nspli
 //   K-B1g warp_bwd_grid_kernel  the forward kernel's structure (persistent CTAs over contiguous ranges of (image, channel)
 //                               planes; [src0 | src1 | gout0 | gout1] of a plane arrive by bulk copies through a 4-stage
 //                               ring; taps / fractions / clip masks of a thread's two pixels in registers): d grid
-//                               accumulates in registers over the channel loop, one add to g_grid per image segment.
+//                               accumulates in registers over the channel loop, one slot per image segment, which
+//                               grid_seg_sum_kernel adds up in a fixed order into g_grid.
 //   K-B1s warp_bwd_src_kernel   d src as a GATHER: persistent CTAs over (image, 8-channel block) units; the image's CSR
 //                               table and the block's gout planes are bulk-copied to shared memory; a thread owns four (two)
 //                               consecutive source pixels and sums  gsrc[s, ch] = sum_e w_e * gout[ch][pix_e]  for the 8
@@ -332,7 +333,21 @@ struct BwdStagedArgs {
   uint32_t s0_bytes, s1_bytes, g_bytes;     // one src0 / src1 / gout plane
   uint32_t in_stage;                        // 128-byte aligned stage size of the d-grid kernel
   unsigned char* csr;                       // [B] blobs of BS_CSR_BYTES
+  float2* seg;                              // [B][seg_max][n] d grid of each image segment (see bwd_cta_of)
+  int seg_max;
 };
+
+// The d-grid kernel's persistent CTA k of `ctas` owns planes [k P / ctas, (k + 1) P / ctas) of the P = B * C (image, channel)
+// planes, so an image is split over consecutive CTAs; the CTA that holds plane x:
+__host__ __device__ __forceinline__ int bwd_cta_of(long long x, int ctas, long long planes) {
+  return (int)(((x + 1) * ctas - 1) / planes);
+}
+static int bwd_grid_ctas(long long planes) { return (int)(planes < sm_count() ? planes : sm_count()); }
+// most CTAs one image is split over: a partial first segment, whole CTA ranges of at least floor(P / ctas) planes, a partial last one
+static int bwd_seg_max(int C, long long planes, int ctas) {
+  const long long whole = C > 2 ? (C - 2) / (planes / ctas) : 0;
+  return (int)(whole + 2 < C ? whole + 2 : C);
+}
 
 // fp64 sampling grid of image b into gridsm (8 lanes per pixel, coalesced float4 rows of pc_score / P_hat); NW warps
 template <int NW>
@@ -637,19 +652,39 @@ __global__ void __launch_bounds__(BS_THREADS, 1) warp_bwd_grid_kernel(BwdStagedA
       __syncwarp();
       if (lane == 0) mbar_arrive(&tail->empty[s]);
     }
-    // d grid of this image segment: chain rule through the un-normalisation (and its clip masks), summed over sources
+    // d grid of this image segment: chain rule through the un-normalisation (and its clip masks), summed over sources, into
+    // the segment's own slot (rank of this CTA among the image's CTAs).  grid_seg_sum_kernel adds the slots in rank order:
+    // float atomics into g_grid summed in arrival order, which is not deterministic once three CTAs share an image (B = 128).
+    const int rank = (int)blockIdx.x - bwd_cta_of((long long)b * C, gridDim.x, a.planes_total);
+    float2* seg = a.seg + ((size_t)b * a.seg_max + rank) * n;
 #pragma unroll
     for (int j = 0; j < BS_PPT; ++j) {
       const int pix = tid + BS_CONSUMERS * j;
       if (pix < n) {
         float ggx = gix0[j] * t0[j].mx, ggy = giy0[j] * t0[j].my;
         if (DUAL) { ggx = __fmaf_rn(gix1[j], t1[j].mx, ggx); ggy = __fmaf_rn(giy1[j], t1[j].my, ggy); }
-        float* gg = p.g_grid + ((size_t)b * n + pix) * 2;
-        atomicAdd(gg, ggx);
-        atomicAdd(gg + 1, ggy);
+        seg[pix] = make_float2(ggx, ggy);
       }
     }
     plane += (c_end - c_begin);
+  }
+}
+
+// g_grid[b][pix] = the image's segment slots summed in rank order (fixed order: deterministic)
+__global__ void __launch_bounds__(256) grid_seg_sum_kernel(BwdStagedArgs a, int ctas) {
+  const WarpParams& p = a.p;
+  const long long total = (long long)p.B * p.n;
+  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < total; i += (long long)gridDim.x * 256) {
+    const int b = (int)(i / p.n), pix = (int)(i - (long long)b * p.n);
+    const long long first = (long long)b * p.C0;
+    const int nseg = bwd_cta_of(first + p.C0 - 1, ctas, a.planes_total) - bwd_cta_of(first, ctas, a.planes_total) + 1;
+    const float2* s = a.seg + (size_t)b * a.seg_max * p.n + pix;
+    float2 acc = s[0];
+    for (int r = 1; r < nseg; ++r) {
+      const float2 v = s[(size_t)r * p.n];
+      acc.x += v.x; acc.y += v.y;
+    }
+    reinterpret_cast<float2*>(p.g_grid)[i] = acc;
   }
 }
 
@@ -827,12 +862,14 @@ static int launch_bwd_t(const tpspp_warp_cfg* cfg, WarpParams p, void* workspace
   if (sizeof(FT) == 4 && cfg->variant != TPSPP_VARIANT_GENERIC && bwd_staged_plan(cfg, p, &sa, &smem_grid, &smem_src)) {
     sa.p.g_grid = p.g_grid;
     sa.csr = reinterpret_cast<unsigned char*>(partial) + align256((size_t)p.B * nsplit * 2 * p.K * sizeof(double));
+    const int grid = bwd_grid_ctas(sa.planes_total);
+    sa.seg = reinterpret_cast<float2*>(sa.csr + align256((size_t)p.B * BS_CSR_BYTES));
+    sa.seg_max = bwd_seg_max(p.C0, sa.planes_total, grid);
     const bool dual = sa.dual != 0;
     auto kgrid = dual ? warp_bwd_grid_kernel<true> : warp_bwd_grid_kernel<false>;
     TPSPP_CHECK_CUDA(cudaFuncSetAttribute(kgrid, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_grid));
     TPSPP_CHECK_CUDA(cudaFuncSetAttribute(warp_bwd_src_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_src));
     TPSPP_CHECK_CUDA(cudaFuncSetAttribute(warp_bwd_csr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bwd_csr_smem()));
-    TPSPP_CHECK_CUDA(cudaMemsetAsync(p.g_grid, 0, (size_t)p.B * n * 2 * sizeof(float), st)); count_launch();
     if (!dual && p.gsrc1) { TPSPP_CHECK_CUDA(cudaMemsetAsync(p.gsrc1, 0, (size_t)p.B * p.C1 * p.H1 * p.W1 * sizeof(FT), st)); count_launch(); }
     const bool want_src = p.gsrc0 != nullptr || (dual && p.gsrc1 != nullptr);
     if (want_src) {
@@ -840,9 +877,10 @@ static int launch_bwd_t(const tpspp_warp_cfg* cfg, WarpParams p, void* workspace
       count_launch();
       TPSPP_CHECK_CUDA(cudaGetLastError());
     }
-    int grid = sm_count();
-    if (grid > sa.planes_total) grid = sa.planes_total;
     kgrid<<<grid, BS_THREADS, smem_grid, st>>>(sa);
+    count_launch();
+    TPSPP_CHECK_CUDA(cudaGetLastError());
+    grid_seg_sum_kernel<<<(unsigned)min(((long long)p.B * n + 255) / 256, 4LL * sm_count()), 256, 0, st>>>(sa, grid);
     count_launch();
     TPSPP_CHECK_CUDA(cudaGetLastError());
     if (want_src) {
@@ -904,9 +942,15 @@ extern "C" size_t tpspp_warp_workspace_bytes(const tpspp_warp_cfg* cfg) {
   if (validate_cfg(cfg) != TPSPP_OK) return 0;
   const size_t n = (size_t)cfg->out_h * cfg->out_w;
   const size_t K = (size_t)cfg->num_fiducial + 3;
+  // the staged kernels' image-segment slots of d grid (only their geometry can use them)
+  size_t seg = 0;
+  if (cfg->mode == TPSPP_MODE_ATTENTION && cfg->num_fiducial == BS_F && cfg->feat_dtype == TPSPP_F32 && cfg->batch > 0) {
+    const long long planes = (long long)cfg->batch * cfg->channels0;
+    seg = (size_t)cfg->batch * bwd_seg_max(cfg->channels0, planes, bwd_grid_ctas(planes)) * n * sizeof(float2);
+  }
   return align256((size_t)cfg->batch * n * 2 * sizeof(float)) +
          align256((size_t)cfg->batch * bwd_nsplit(cfg) * 2 * K * sizeof(double)) +
-         align256((size_t)cfg->batch * BS_CSR_BYTES) /* per-image scatter tables of the staged kernels */ + 256;
+         align256((size_t)cfg->batch * BS_CSR_BYTES) /* per-image scatter tables of the staged kernels */ + align256(seg) + 256;
 }
 
 extern "C" int tpspp_warp_bwd(const tpspp_warp_cfg* cfg, const void* src0, const void* src1,
