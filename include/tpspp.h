@@ -388,6 +388,38 @@ typedef struct tpspp_attn_encode_cfg {
 TPSPP_API int tpspp_attn_encode(const tpspp_attn_encode_cfg* cfg, const float* q, const float* k, const float* v,
                                 const int32_t* kv_lens /* [batch] device pointer or NULL */, float* out, tpspp_stream_t stream);
 
+/* ---- Training attention: forward and backward of the NRTR encoder's self-attention, the decoder's causal self-attention and
+ * its cross-attention over the encoder memory, with the reference's attention dropout (ScaledDotProductAttention,
+ * common/modules/transformer_module.py:24-34: P_drop = P * keep / (1 - dropout_p)).
+ *   S[b,h,i,j] = (q[b,i,h,:] / temperature) . k[b,j,h,:]   over keys j < len(b) and, with `causal`, j <= i
+ *   out[b,i,h,:] = sum_j softmax_j(S)[b,h,i,j] keep(b,h,i,j) / (1 - dropout_p) v[b,j,h,:]      for every i < len_q
+ * q [batch*len_q, heads*64] rows q_stride floats apart; k / v [batch*len_k, heads*64] rows kv_stride floats apart (q, k, v may be
+ * column slices of one fused q|k|v projection, k / v of one fused k|v projection); out [batch*len_q, heads*64] row-major;
+ * lse [batch, heads, len_q]: the log-sum-exp of each row of S over its valid keys, which the backward pass recomputes P from.
+ * len(b) = kv_lens[b] (device int32, >= 1; the caller checks it) or len_k.  Every query row is computed, also i >= len(b).
+ * keep(b,h,i,j) is bit r = i mod 4 of Philox4x32-10 (counter (j, i / 4, h, b), key = the 64-bit seed at seed_ptr) compared with
+ * dropout_p * 2^32: no mask is stored and the backward pass regenerates it.  seed_ptr is a device pointer (read by the kernels,
+ * so a seed drawn on the device needs no host sync, and with device-resident kv_lens the calls can be captured in a graph); with dropout_p = 0 nothing is
+ * drawn and seed_ptr may be NULL.  1 <= len_q, len_k <= 256; fp32 on CUDA cores; pointers 16-byte aligned. */
+typedef struct tpspp_attn_train_cfg {
+  int32_t batch, heads, head_dim;   /* batch <= 65535; head_dim = 64                                        */
+  int32_t len_q, len_k;             /* queries / keys per image, 1..256                                     */
+  float temperature;                /* d_k ** 0.5 in the reference                                          */
+  int32_t causal;                   /* 1: key j is also masked for query i < j (decoder self-attention)     */
+  float dropout_p;                  /* attention dropout, 0 <= p < 1                                        */
+  int32_t q_stride, kv_stride;      /* floats between consecutive rows of q (and gq) / of k, v (and gk, gv); 0 = heads*64; multiples of 4 */
+} tpspp_attn_train_cfg;
+TPSPP_API int tpspp_attn_train_fwd(const tpspp_attn_train_cfg* cfg, const float* q, const float* k, const float* v,
+                                   const int32_t* kv_lens /* [batch] device pointer or NULL */, const uint64_t* seed_ptr,
+                                   float* out, float* lse, tpspp_stream_t stream);
+/* dq / dk / dv from gout (= dL/dout) by recomputation: P = exp(S - lse), D = rowsum(gout * out), dS = P * (dP - D) with
+ * dP = (gout . v^T) * keep / (1 - p).  gq has q's row stride, gk / gv kv_stride (they may be column slices of one fused gradient
+ * buffer); every row is written (zeros for keys j >= len(b)).  No floating-point atomics: query-block CTAs write dq, key-block
+ * CTAs dk and dv, so two calls on the same inputs give the same bits. */
+TPSPP_API int tpspp_attn_train_bwd(const tpspp_attn_train_cfg* cfg, const float* q, const float* k, const float* v, const float* out,
+                                   const float* gout, const float* lse, const int32_t* kv_lens, const uint64_t* seed_ptr,
+                                   float* gq, float* gk, float* gv, tpspp_stream_t stream);
+
 /* ---- Text-recognition test pipeline: mmocr 0.4 ResizeOCR -> ToTensorOCR -> NormalizeOCR (reference
  * datasets/pipelines/ocr_transforms.py:67-130) for a whole ragged batch of uint8 images in one launch.
  *   packed  uint8 HWC images, 3 channels in the caller's channel order (no BGR/RGB swap), one after the other

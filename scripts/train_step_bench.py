@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Training-step timing of the rectifier (BASELINE config 3, rectifier part): forward + backward +
-one flat-bucket NCCL all-reduce + Adam, batch 128 per GPU.  NRTR itself is out of scope (SURVEY 8f), so
-the loss is a synthetic regression on `output`.  Launch: python scripts/train_step_bench.py  or
+one flat-bucket NCCL all-reduce + Adam, batch 128 per GPU.  The loss is a synthetic regression on `output`; the whole
+recogniser's step (NRTR.forward_train, TFLoss) is scripts/nrtr_train_step_bench.py.  Launch: python scripts/train_step_bench.py  or
 python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 scripts/train_step_bench.py"""
 import json
 import os

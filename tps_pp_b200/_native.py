@@ -69,6 +69,12 @@ class AttnEncodeCfg(Structure):
                 ("row_stride", c_int32)]
 
 
+class AttnTrainCfg(Structure):
+    """Mirror of ``tpspp_attn_train_cfg`` (include/tpspp.h)."""
+    _fields_ = [("batch", c_int32), ("heads", c_int32), ("head_dim", c_int32), ("len_q", c_int32), ("len_k", c_int32),
+                ("temperature", c_float), ("causal", c_int32), ("dropout_p", c_float), ("q_stride", c_int32), ("kv_stride", c_int32)]
+
+
 class OcrPrepCfg(Structure):
     """Mirror of ``tpspp_ocr_prep_cfg`` (include/tpspp.h)."""
     _fields_ = [("n", c_int32), ("out_h", c_int32), ("out_w", c_int32), ("mean", c_float * 3), ("std", c_float * 3),
@@ -119,6 +125,8 @@ _SIGNATURES = {
     "tpspp_locnet_fwd": (c_int, [POINTER(LocnetCfg), c_void_p, POINTER(c_void_p), c_void_p, c_void_p, c_void_p]),
     "tpspp_attn_decode": (c_int, [POINTER(AttnCfg)] + [c_void_p] * 8),
     "tpspp_attn_encode": (c_int, [POINTER(AttnEncodeCfg)] + [c_void_p] * 6),
+    "tpspp_attn_train_fwd": (c_int, [POINTER(AttnTrainCfg)] + [c_void_p] * 8),
+    "tpspp_attn_train_bwd": (c_int, [POINTER(AttnTrainCfg)] + [c_void_p] * 12),
     "tpspp_ocr_prep": (c_int, [POINTER(OcrPrepCfg)] + [c_void_p] * 4),
     "tpspp_linear_fwd_ex": (c_int, [POINTER(LinearCfg)] + [c_void_p] * 4 + [c_int32] + [c_void_p] * 3),
     "tpspp_linear_ln_fwd": (c_int, [POINTER(LinearCfg)] + [c_void_p] * 4 + [c_int32] + [c_void_p] * 3 + [ctypes.c_float] + [c_void_p] * 3),

@@ -720,3 +720,137 @@ def ocr_prep(packed: torch.Tensor, desc, out_h: int, out_w: int, mean, std, pad_
     with torch.cuda.device(packed.device):
         N.check(N.lib().tpspp_ocr_prep(ctypes.byref(cfg), _ptr(packed), _ptr(desc_dev), _ptr(out), _stream(packed)), "tpspp_ocr_prep")
     return out
+
+
+def _fused_source(t: torch.Tensor):
+    """``(base, column offset)`` when ``t`` is a column block of a contiguous 2-D tensor (a slice of a fused projection), else
+    ``(t, 0)`` -- so that the attention's gradient lands in the fused projection's gradient without a ``torch.cat``."""
+    b = t._base
+    # the base stands in for t only when autograd treats them alike (a slice made a leaf by requires_grad_() has a base
+    # that does not require grad: its gradient must stay with the slice)
+    if (b is not None and b.requires_grad == t.requires_grad and b.dim() == 2 and b.is_contiguous() and t.dim() == 2 and t.stride(1) == 1
+            and t.shape[0] == b.shape[0] and (t.shape[0] <= 1 or t.stride(0) == b.stride(0))):
+        off = t.storage_offset() - b.storage_offset()
+        if 0 <= off and off + t.shape[1] <= b.shape[1]:
+            return b, off
+    return t, 0
+
+
+class AttnLengths:
+    """Key lengths of an attention call checked on the host (each in [1, len_k], ``ValueError`` otherwise: the reference's soft-max
+    over no key gives NaN rows) and uploaded once, so several ``attention`` calls share them without a read-back or a copy."""
+
+    def __init__(self, lens, len_k: int, device):
+        if isinstance(lens, torch.Tensor):
+            if lens.dtype not in (torch.int32, torch.int64) or lens.dim() != 1:
+                raise RuntimeError("tps_pp_b200: kv_lens must be a 1-D integer tensor or a sequence of ints")
+            host = lens.tolist()                     # a device tensor is read back once: the lengths are checked before any launch
+        else:
+            host = [int(x) for x in lens]
+        bad = [x for x in host if not 1 <= x <= int(len_k)]
+        if bad:
+            raise ValueError(f"tps_pp_b200: attention key lengths must lie in [1, {len_k}], got {bad[0]} (an image without a valid "
+                             "key has no soft-max: the reference gives NaN rows)")
+        self.host, self.len_k = tuple(host), int(len_k)
+        self.dev = torch.tensor(host, dtype=torch.int32).to(device, non_blocking=True)
+
+
+class _Attention(torch.autograd.Function):
+    """Multi-head attention with native forward AND backward (``tpspp_attn_train_fwd`` / ``tpspp_attn_train_bwd``).  The inputs
+    are the tensors q / k / v are column blocks of (``srcs``; ``where[n] = (source index, column offset)``); the gradient of
+    each source is written by the kernels in place of its column blocks.  ``calls`` counts the forward launches."""
+
+    calls = 0
+
+    @staticmethod
+    def forward(ctx, meta, *srcs):
+        where, cfg_args, kv_lens = meta
+        q, k, v = [srcs[s][:, off:off + cfg_args[1] * 64] for s, off in where]
+        cfg = N.AttnTrainCfg(*cfg_args[:8], int(srcs[where[0][0]].stride(0)), int(srcs[where[1][0]].stride(0)))
+        rows_q, d = cfg.batch * cfg.len_q, cfg.heads * 64
+        out = torch.empty((rows_q, d), dtype=torch.float32, device=q.device)
+        lse = torch.empty((cfg.batch, cfg.heads, cfg.len_q), dtype=torch.float32, device=q.device)
+        _Attention.calls += 1
+        seed = None
+        if cfg.dropout_p > 0:
+            # drawn on the device from torch's CUDA generator: torch.manual_seed reproduces it, no host sync
+            seed = torch.randint(0, 2 ** 62, (1,), dtype=torch.int64, device=q.device)
+        with torch.cuda.device(q.device):
+            N.check(N.lib().tpspp_attn_train_fwd(ctypes.byref(cfg), _ptr(q), _ptr(k), _ptr(v), _ptr(kv_lens), _ptr(seed), _ptr(out),
+                                                 _ptr(lse), _stream(q)), "tpspp_attn_train_fwd")
+        ctx.save_for_backward(out, lse, *srcs)
+        ctx.meta = (where, cfg_args, kv_lens, seed)
+        ctx.mark_non_differentiable(lse)
+        return out, lse
+
+    @staticmethod
+    def backward(ctx, gout, _glse):
+        out, lse, *srcs = ctx.saved_tensors
+        where, cfg_args, kv_lens, seed = ctx.meta
+        d = cfg_args[1] * 64
+        covered = [0] * len(srcs)
+        for s, _ in where:
+            covered[s] += d
+        grads = [torch.empty_like(t) if covered[i] == t.shape[1] else torch.zeros_like(t) for i, t in enumerate(srcs)]
+        q, k, v = [srcs[s][:, off:off + d] for s, off in where]
+        gq, gk, gv = [grads[s][:, off:off + d] for s, off in where]
+        cfg = N.AttnTrainCfg(*cfg_args[:8], int(srcs[where[0][0]].stride(0)), int(srcs[where[1][0]].stride(0)))
+        gout = gout.contiguous()
+        with torch.cuda.device(out.device):
+            N.check(N.lib().tpspp_attn_train_bwd(ctypes.byref(cfg), _ptr(q), _ptr(k), _ptr(v), _ptr(out), _ptr(gout), _ptr(lse),
+                                                 _ptr(kv_lens), _ptr(seed), _ptr(gq), _ptr(gk), _ptr(gv), _stream(out)),
+                    "tpspp_attn_train_bwd")
+        return (None, *grads)
+
+
+def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, len_q: int, len_k: int, temperature: float,
+              kv_lens=None, causal: bool = False, dropout_p: float = 0.0) -> torch.Tensor:
+    """Multi-head attention over whole sequences with native forward and backward (``tpspp_attn_train_fwd`` / ``_bwd``),
+    differentiable in q, k and v: the reference's ``MultiHeadAttention`` core (transformer_module.py:24-34,74-98) between the
+    projections, with its attention dropout.
+
+    q [B*len_q, heads*64], k / v [B*len_k, heads*64] token-major fp32 -> out [B*len_q, heads*64].  Image b's query i attends to its
+    keys j < kv_lens[b] (all len_k without ``kv_lens``) and, with ``causal``, j <= i; ``dropout_p`` > 0 drops probabilities with a
+    seed drawn from torch's CUDA generator.  ``kv_lens``: an :class:`AttnLengths` (checked and uploaded once, for calls that
+    share lengths), or host ints (a list or CPU tensor; a CUDA tensor is read back once) each in [1, len_k] -- ``ValueError``
+    otherwise.  q / k / v may be column slices of one fused projection (k / v must share a row stride):
+    their gradients are then written straight into the fused projection's gradient.  1 <= len_q, len_k <= 256."""
+    for nm, t in (("q", q), ("k", k), ("v", v)):
+        _require_cuda(nm, t, torch.float32)
+    len_q, len_k, heads = int(len_q), int(len_k), int(heads)
+    d = heads * 64
+    if not (1 <= len_q <= 256 and 1 <= len_k <= 256):
+        raise ValueError(f"tps_pp_b200: attention takes 1 <= len_q, len_k <= 256, got {len_q}, {len_k}")
+    if not 0.0 <= float(dropout_p) < 1.0:
+        raise ValueError(f"tps_pp_b200: attention dropout_p must lie in [0, 1), got {dropout_p}")
+    if q.dim() != 2 or q.shape[1] != d or q.shape[0] % len_q:
+        raise RuntimeError(f"tps_pp_b200: attention q must be [B*{len_q}, {d}] for {heads} heads, got {tuple(q.shape)}")
+    b = q.shape[0] // len_q
+    for nm, t, L in (("q", q, len_q), ("k", k, len_k), ("v", v, len_k)):
+        if t.dim() != 2 or t.shape != (b * L, d) or t.stride(1) != 1 or t.device != q.device:
+            raise RuntimeError(f"tps_pp_b200: attention `{nm}` must be [{b * L}, {d}] on {q.device} with unit stride along the features")
+    srcs, where = [], []
+    for t in (q, k, v):
+        base, off = _fused_source(t)
+        s = next((i for i, x in enumerate(srcs) if x is base), None)
+        # the same columns used twice (attention(h, h, h)): a separate gradient buffer, summed by autograd
+        if s is not None and any(ws == s and wo == off for ws, wo in where):
+            s = None
+        if s is None:
+            if base is t and t.stride(0) != d and t.shape[0] > 1:
+                base = t.contiguous()
+            srcs.append(base)
+            s = len(srcs) - 1
+        where.append((s, off))
+    if srcs[where[1][0]].stride(0) != srcs[where[2][0]].stride(0):
+        raise RuntimeError("tps_pp_b200: attention k / v must share one row stride")
+    lens = None
+    if kv_lens is not None:
+        if not isinstance(kv_lens, AttnLengths):
+            kv_lens = AttnLengths(kv_lens, len_k, q.device)
+        if len(kv_lens.host) != b or kv_lens.len_k > len_k or kv_lens.dev.device != q.device:
+            raise RuntimeError(f"tps_pp_b200: kv_lens must have one entry per image ({b}), each <= len_k = {len_k}, on {q.device}")
+        lens = kv_lens.dev
+    cfg_args = (b, heads, 64, len_q, len_k, float(temperature), 1 if causal else 0, float(dropout_p))
+    out, _ = _Attention.apply((tuple(where), cfg_args, lens), *srcs)
+    return out

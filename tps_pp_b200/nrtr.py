@@ -16,7 +16,8 @@ processes ONE token per image -- dense layers on the tcgen05 3xTF32 kernels (``t
 caches in ``tpspp_attn_decode``; residual adds, GELU and the LayerNorm in front of the next sub-layer run in the dense layers'
 epilogues (``tpspp_linear_ln_fwd``); the embedding gather, the first LayerNorm of a step and the soft-max are torch ops.
 Position ``t`` of the causal, pad-masked reference attends exactly to tokens ``0..t``, so the results are the reference's
-up to fp32 summation order.  ``forward_train`` and ``forward_test_library`` (the reference's algorithm, for A/B) run torch ops.
+up to fp32 summation order.  ``forward_train`` and ``forward_test_library`` (the reference's algorithm, for A/B) run torch ops; the recogniser's training
+path is ``nrtr_train.decoder_train`` (native attention and dense layers, forward and backward, with the reference's dropout).
 """
 from __future__ import annotations
 
@@ -279,8 +280,9 @@ class NRTREncoder(_BaseModule):
     the next layer's ``norm1`` (after the last layer: the final ``layer_norm``) -- the tcgen05 3xTF32 dense kernels of
     ``NRTRDecoder``.  ``forward_library`` is the reference algorithm on torch ops; ``forward`` uses it while autograd records,
     in training mode, for head sizes other than 64 or model widths that are not a multiple of 128, and for an image whose
-    valid length is 0 (the reference's soft-max over no key: NaN rows).  Dropout is the identity in eval mode and is not
-    applied by either path (training runs in mmocr)."""
+    valid length is 0 (the reference's soft-max over no key: NaN rows).  Neither path applies dropout (the identity in eval
+    mode); ``nrtr_train.encoder_train`` is the training forward with the reference's dropout (``p = dropout``) on native
+    forward and backward kernels, which ``NRTR.forward_train`` uses."""
 
     def __init__(self, n_layers=6, n_head=8, d_k=64, d_v=64, d_model=512, d_inner=256, dropout=0.1, init_cfg=None, **kwargs):
         super().__init__(init_cfg=init_cfg)
@@ -294,6 +296,7 @@ class NRTREncoder(_BaseModule):
         if act_cfg is not None and dict(act_cfg) not in (dict(type="mmcv.GELU"), dict(type="GELU")):
             raise ValueError(f"tps_pp_b200.NRTREncoder implements the GELU feed-forward only, got act_cfg={act_cfg!r}")
         self.n_layers, self.n_head, self.d_k, self.d_v, self.d_model = n_layers, n_head, d_k, d_v, d_model
+        self.dropout = dropout            # applied by nrtr_train.encoder_train in training mode
         layers = []
         for _ in range(n_layers):
             lyr = nn.Module()

@@ -5,7 +5,9 @@ dictionary and the decode of class probabilities into strings.  ``NRTR`` (regist
 recognizer/nrtr.py over ``EncodeDecodeRecognizer``, recognizer/encode_decode_recognizer.py): ``backbone`` (with ``tpsnet``
 called mid-way), ``encoder``, ``decoder`` and ``label_convertor`` built from config dicts, under the reference's sub-module
 names so that ``backbone.*`` / ``tpsnet.*`` / ``encoder.*`` / ``decoder.*`` checkpoint keys load with ``strict=True``.
-Inference only: ``simple_test`` (encode_decode_recognizer.py:184-225); training runs in mmocr.
+Inference: ``simple_test`` (encode_decode_recognizer.py:184-225).  Training: ``forward_train`` (encode_decode_recognizer.py:
+``forward_train``) -- the labels through ``AttnConvertor.str2tensor``, the encoder and the teacher-forced decoder on native
+attention and dense kernels (``nrtr_train``), ``TFLoss`` (registry ``LOSSES``; reference losses/ce_loss.py).
 """
 from __future__ import annotations
 
@@ -14,7 +16,11 @@ from typing import List, Optional, Sequence
 import torch
 import torch.nn as nn
 
-from .registry import CONVERTORS, RECOGNIZERS, build_backbone, build_convertor, build_decoder, build_encoder, build_preprocessor
+from . import functional as TF
+from . import nrtr_train
+from .nrtr import NRTRDecoder, NRTREncoder, valid_lengths
+from .registry import (CONVERTORS, LOSSES, RECOGNIZERS, build_backbone, build_convertor, build_decoder, build_encoder, build_loss,
+                       build_preprocessor)
 
 DICT36 = tuple("0123456789abcdefghijklmnopqrstuvwxyz")
 DICT90 = tuple("0123456789abcdefghijklmnopqrstuvwxyz"
@@ -78,6 +84,63 @@ class AttnConvertor:
     def idx2str(self, indexes: Sequence[Sequence[int]]) -> List[str]:
         return ["".join(self.idx2char[i] for i in index) for index in indexes]
 
+    def str2idx(self, strings: Sequence[str]) -> List[List[int]]:
+        """convertors/base.py ``str2idx``: each string (lower-cased with ``lower``) to its character indexes; a character outside
+        the dictionary is ``<UKN>``, or raises ``ValueError`` without ``with_unknown``."""
+        if not isinstance(strings, (list, tuple)) or not all(isinstance(s, str) for s in strings):
+            raise TypeError("tps_pp_b200.AttnConvertor.str2idx takes a list of strings")
+        indexes = []
+        for string in strings:
+            if self.lower:
+                string = string.lower()
+            index = []
+            for char in string:
+                i = self.char2idx.get(char, self.unknown_idx)
+                if i is None:
+                    raise ValueError(f"tps_pp_b200.AttnConvertor: character {char!r} is not in the dictionary; use a dictionary that "
+                                     "holds it or with_unknown=True")
+                index.append(i)
+            indexes.append(index)
+        return indexes
+
+    def str2tensor(self, strings: Sequence[str]):
+        """convertors/attn.py ``str2tensor``: ``targets`` (per string its character indexes, LongTensor) and ``padded_targets``
+        [N, max_seq_len] -- ``[start, chars..., end]`` filled up with ``padding_idx``, cut at ``max_seq_len`` when longer."""
+        targets, padded = [], []
+        for index in self.str2idx(strings):
+            targets.append(torch.LongTensor(index))
+            seq = [self.start_idx] + index + [self.end_idx]
+            row = torch.full((self.max_seq_len,), self.padding_idx, dtype=torch.long)
+            seq = seq[:self.max_seq_len]
+            row[:len(seq)] = torch.LongTensor(seq)
+            padded.append(row)
+        return dict(targets=targets, padded_targets=torch.stack(padded, 0))
+
+
+@LOSSES.register_module()
+class TFLoss(nn.Module):
+    """mmocr 0.4 ``TFLoss`` (losses/ce_loss.py): the cross-entropy of ``outputs[:, :-1]`` against ``padded_targets[:, 1:]``
+    (each step predicts the next token), flattened, with ``reduction='none'`` -- one loss per (image, step), 0 where the target is
+    ``ignore_index`` (the recogniser sets it to the padding index).  Returns ``dict(loss_ce=...)``."""
+
+    def __init__(self, ignore_index=-1, reduction="none", flatten=True, **kwargs):
+        super().__init__()
+        if not isinstance(flatten, bool):
+            raise TypeError("tps_pp_b200.TFLoss: flatten must be a bool")
+        self.flatten = flatten
+        self.loss_ce = nn.CrossEntropyLoss(ignore_index=ignore_index, reduction=reduction)
+
+    def format(self, outputs, targets_dict):
+        outputs = outputs[:, :-1, :].contiguous()
+        targets = targets_dict["padded_targets"][:, 1:].contiguous()
+        if self.flatten:
+            return outputs.view(-1, outputs.size(-1)), targets.view(-1)
+        return outputs.permute(0, 2, 1).contiguous(), targets
+
+    def forward(self, outputs, targets_dict, img_metas=None):
+        outputs, targets = self.format(outputs, targets_dict)
+        return dict(loss_ce=self.loss_ce(outputs, targets.to(outputs.device)))
+
 
 @RECOGNIZERS.register_module()
 class NRTR(nn.Module):
@@ -99,6 +162,9 @@ class NRTR(nn.Module):
                                           max_seq_len=max_seq_len))
         self.loss_cfg, self.train_cfg, self.test_cfg, self.init_cfg = loss, train_cfg, test_cfg, init_cfg
         self.max_seq_len = max_seq_len
+        # as EncodeDecodeRecognizer.__init__: the loss ignores the padding index
+        self.loss = build_loss(dict(loss if loss is not None else dict(type="TFLoss"), ignore_index=self.label_convertor.padding_idx))
+        self.last_train_native = None
 
     def extract_feat(self, img):
         """encode_decode_recognizer.py: optional preprocessor, then the backbone with the rectifier called mid-way."""
@@ -118,8 +184,36 @@ class NRTR(nn.Module):
         strings = self.label_convertor.idx2str(indexes)
         return [dict(text=s, score=sc) for s, sc in zip(strings, scores)]
 
+    def forward_train(self, img, img_metas):
+        """encode_decode_recognizer.py ``forward_train``: images [N, 3, H, W] and one meta per image with its ground-truth
+        ``text`` -> ``dict(loss_ce=[N * (max_seq_len - 1)] per-step losses)``.  Each image's ``valid_ratio`` is
+        ``resize_shape[1] / W`` where the meta has ``resize_shape``, else its ``valid_ratio`` (default 1.0).  The backbone runs in
+        its training form (``TPS_PP`` on its native training path); the encoder and the teacher-forced decoder run on native
+        attention and dense kernels, forward and backward (``nrtr_train``); ``last_train_native`` records whether every attention
+        call of both halves ran the native kernels."""
+        if img_metas is None or any(not isinstance(m, dict) or "text" not in m for m in img_metas):
+            raise RuntimeError("tps_pp_b200.NRTR.forward_train: each image's ground-truth `text` must come in img_metas, as mmocr's "
+                               "training pipeline provides it")
+        if len(img_metas) != img.shape[0]:
+            raise ValueError(f"tps_pp_b200.NRTR.forward_train: {img.shape[0]} images but {len(img_metas)} img_metas")
+        if not isinstance(self.encoder, NRTREncoder) or not isinstance(self.decoder, NRTRDecoder):
+            raise RuntimeError("tps_pp_b200.NRTR.forward_train needs the NRTREncoder and NRTRDecoder of this package")
+        self.last_train_native = False
+        calls = TF._Attention.calls
+        metas = []
+        for m in img_metas:
+            ratio = m["resize_shape"][1] / img.shape[-1] if "resize_shape" in m else m.get("valid_ratio", 1.0)
+            metas.append(dict(m, valid_ratio=ratio))
+        feat = self.extract_feat(img)
+        targets_dict = self.label_convertor.str2tensor([m["text"] for m in metas])
+        lens = valid_lengths(feat.shape[2] * feat.shape[3], metas)
+        out_enc = nrtr_train.encoder_train(self.encoder, feat, lens)
+        out_dec = nrtr_train.decoder_train(self.decoder, targets_dict["padded_targets"], out_enc, lens)
+        # every attention call of both halves ran the native kernels: one per encoder layer, two per decoder layer
+        self.last_train_native = TF._Attention.calls - calls == len(self.encoder.layer_stack) + 2 * len(self.decoder.layer_stack)
+        return self.loss(out_dec, targets_dict, metas)
+
     def forward(self, img, img_metas=None, return_loss=False, **kwargs):
         if return_loss:
-            raise RuntimeError("tps_pp_b200.NRTR is the inference recogniser: training (return_loss=True) runs in mmocr, with "
-                               "the drop-in modules registered by tps_pp_b200.register_into_mmocr()")
+            return self.forward_train(img, img_metas)
         return self.simple_test(img, img_metas, **kwargs)

@@ -47,6 +47,8 @@ DECODERS = Registry("decoder")
 ENCODERS = Registry("encoder")
 CONVERTORS = Registry("convertor")
 RECOGNIZERS = Registry("recognizer")
+# the recogniser's losses (TFLoss); not registered into mmocr, which has its own
+LOSSES = Registry("loss")
 # the batched GPU test pipeline (tps_pp_b200/pipeline.py); not registered into mmocr: its transforms run per image on the host
 PIPELINES = Registry("pipeline")
 
@@ -75,6 +77,11 @@ def build_encoder(cfg):
 def build_convertor(cfg):
     """reference mmocr/models/builder.py (``CONVERTORS``); used for ``label_convertor`` at recognizer/encode_decode_recognizer.py."""
     return CONVERTORS.build(cfg)
+
+
+def build_loss(cfg):
+    """reference mmocr/models/builder.py (``LOSSES``); used for ``loss`` at recognizer/encode_decode_recognizer.py."""
+    return LOSSES.build(cfg)
 
 
 def build_recognizer(cfg):
