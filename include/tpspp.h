@@ -423,21 +423,25 @@ TPSPP_API int tpspp_attn_train_bwd(const tpspp_attn_train_cfg* cfg, const float*
 /* ---- Text-recognition test pipeline: mmocr 0.4 ResizeOCR -> ToTensorOCR -> NormalizeOCR (reference
  * datasets/pipelines/ocr_transforms.py:67-130) for a whole ragged batch of uint8 images in one launch.
  *   packed  uint8 HWC images, 3 channels in the caller's channel order (no BGR/RGB swap), one after the other
- *   desc    [n][4] int64 device array: byte offset of the image in `packed`, h, w, resize_w (the width ResizeOCR chose)
+ *   desc    [n][4] int64 device array: byte offset of the image in `packed`, h, w, resize_w (the width ResizeOCR chose);
+ *           with TPSPP_OCR_FLAG_ROTATED [n][5]: the same four (h, w of the STORED image), then k, the number of quarter turns
+ *           counter-clockwise (np.rot90(img, k)); the kernel uses k & 3.  Several descriptors may share one offset.
  *   out     [n, 3, out_h, out_w] fp32 NCHW
  * Pixel (c, y, x) of image i: x < resize_w: cv2.resize(img, (resize_w, out_h), INTER_LINEAR) on uint8 (OpenCV's fixed-point
- * arithmetic, bit for bit); x >= resize_w: pad_value (mmcv.impad).  Then ((float)u8 / 255 - mean[c]) / std[c] in fp32 with
+ * arithmetic, bit for bit), where img is np.rot90(stored, k) with TPSPP_OCR_FLAG_ROTATED (w x h for odd k) and the stored
+ * image otherwise; x >= resize_w: pad_value (mmcv.impad).  Then ((float)u8 / 255 - mean[c]) / std[c] in fp32 with
  * IEEE divisions (torchvision to_tensor + normalize).  The library cannot read the descriptors without a host sync, so it does
  * not validate them; every read of `packed` is bounded by packed_bytes, so a corrupt descriptor gives wrong pixels but never an
  * out-of-range access.  The Python wrapper (tps_pp_b200/functional.py::ocr_prep) checks descriptors on the host. */
 typedef struct tpspp_ocr_prep_cfg {
-  int32_t n;                /* images                                                               */
+  int32_t n;                /* images (descriptors)                                                 */
   int32_t out_h, out_w;     /* ResizeOCR height, max_width                                          */
   float mean[3], std[3];    /* NormalizeOCR, per channel of the caller's order; std != 0            */
   int32_t pad_value;        /* ResizeOCR img_pad_value, uint8 domain [0, 255]                       */
-  int32_t flags;            /* 0 (reserved)                                                         */
+  int32_t flags;            /* 0 or TPSPP_OCR_FLAG_ROTATED; any other bit is rejected               */
   int64_t packed_bytes;     /* size of `packed`: every read stays below it                          */
 } tpspp_ocr_prep_cfg;
+enum { TPSPP_OCR_FLAG_ROTATED = 2 };  /* desc is [n][5]: rotation test-time augmentation (mmocr MultiRotateAugOCR) */
 TPSPP_API int tpspp_ocr_prep(const tpspp_ocr_prep_cfg* cfg, const uint8_t* packed, const int64_t* desc, float* out,
                              tpspp_stream_t stream);
 

@@ -95,6 +95,7 @@ HEAD_FLAG_UNFUSED_SCORE = 4
 HEAD_FLAG_TF32X3_CONV = 8
 HEAD_FLAG_FEATGRID_BF16 = 16
 LINEAR_FLAG_WEIGHTS_CACHED = 1
+OCR_FLAG_ROTATED = 2
 ACT_NONE, ACT_GELU = 0, 1
 ABI_VERSION = 2
 P_COUNT = 58

@@ -37,7 +37,11 @@ def init_recognizer(config, checkpoint=None, device="cuda"):
 
 def model_inference(model, imgs, batch_size: int = 256):
     """One image (uint8 [H, W, 3] array or path) -> ``dict(text, score)``; a list of them -> a list of such dicts.  Works in
-    chunks of at most ``batch_size`` images under ``torch.no_grad()``; every input is checked before the first chunk runs."""
+    chunks of at most ``batch_size`` images under ``torch.no_grad()``; every input is checked before the first chunk runs.
+
+    With a ``MultiRotateAugOCR`` test pipeline, ``batch_size`` bounds the rotations a chunk holds: a chunk takes whole images
+    while their rotations fit, so ``batch_size`` must be at least the number of distinct rotate degrees.  Each image's
+    readings are merged by ``model.merge_aug_results`` into ``dict(text, score)`` with a float ``score``."""
     if int(batch_size) < 1:
         raise ValueError(f"tps_pp_b200.model_inference: batch_size must be >= 1, got {batch_size}")
     single = isinstance(imgs, (np.ndarray, str, os.PathLike))
@@ -49,9 +53,36 @@ def model_inference(model, imgs, batch_size: int = 256):
     pipeline = getattr(model, "test_pipeline", None)
     if pipeline is None:
         raise ValueError("tps_pp_b200.model_inference: the model has no test_pipeline (build it with init_recognizer)")
+    rotate = getattr(pipeline, "rotate", None)
+    if rotate is not None and int(batch_size) < len(set(rotate.rotate_degrees)):
+        raise ValueError(f"tps_pp_b200.model_inference: batch_size {batch_size} is smaller than the {len(set(rotate.rotate_degrees))} "
+                         "rotations MultiRotateAugOCR reads a tall image in")
     results = []
     with torch.no_grad():
-        for s in range(0, len(items), int(batch_size)):
-            img, metas = pipeline(items[s:s + int(batch_size)])
-            results += model.simple_test(img, metas)
+        if rotate is None:
+            for s in range(0, len(items), int(batch_size)):
+                img, metas = pipeline(items[s:s + int(batch_size)])
+                results += model.simple_test(img, metas)
+        else:
+            chunk, rows = [], 0
+            for i, x in enumerate(items):
+                img, fname = pipeline.load.load(x, i)
+                n = len(rotate.degrees(*img.shape[:2]))
+                if rows + n > int(batch_size):
+                    results += _aug_chunk(model, pipeline, chunk)
+                    chunk, rows = [], 0
+                chunk.append((img, fname))
+                rows += n
+            results += _aug_chunk(model, pipeline, chunk)
     return results[0] if single else results
+
+
+def _aug_chunk(model, pipeline, loaded):
+    """Whole images through the rotating pipeline and one ``simple_test``, then one merged result per image."""
+    img, metas = pipeline.prepare(loaded)
+    flat = model.simple_test(img, [m for group in metas for m in group])
+    out, s = [], 0
+    for group in metas:
+        out += model.merge_aug_results(flat[s:s + len(group)])
+        s += len(group)
+    return out

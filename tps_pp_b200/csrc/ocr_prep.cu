@@ -11,6 +11,14 @@
 // explicit _rn intrinsics so that no multiply-add is contracted into an FMA: OpenCV's x86 build rounds each step.
 // The rows of the fp32 output are written coalesced; the source bytes are gathered through L1 and every read is bounded by
 // cfg.packed_bytes (the descriptors are not validated on the device).
+// With TPSPP_OCR_FLAG_ROTATED (mmocr's MultiRotateAugOCR) a descriptor has a fifth field k, and the image resampled is
+// np.rot90(S, k & 3) of the stored H x W image S (W x H for odd k).  The arithmetic above runs on the rotated frame's sizes, and
+// each tap (i, j) of the rotated frame is read at its stored address off + 3 * (base + i * si + j * sj):
+//   k = 0: S[i, j]          si =  W, sj =  1, base = 0
+//   k = 1: S[j, W-1-i]      si = -1, sj =  W, base = W - 1
+//   k = 2: S[H-1-i, W-1-j]  si = -W, sj = -1, base = H W - 1
+//   k = 3: S[H-1-j, i]      si =  1, sj = -W, base = (H - 1) W
+// so several descriptors can point at the same packed bytes.  The flag-less kernel is the ROTATED = false instantiation.
 #include "common.cuh"
 
 namespace tpspp {
@@ -38,20 +46,38 @@ __device__ __forceinline__ float op_norm(int u, float mean, float std_) {
   return __fdiv_rn(__fsub_rn(__fdiv_rn((float)u, 255.f), mean), std_);
 }
 
+template <bool ROTATED>
 __global__ void __launch_bounds__(OP_THREADS) ocr_prep_kernel(const uint8_t* __restrict__ packed, const long long* __restrict__ desc,
                                                               float* __restrict__ out, const OcrPrepArgs a) {
+  constexpr int NF = ROTATED ? 5 : 4;       // descriptor fields
   const int img = blockIdx.x, y = blockIdx.y;
-  const long long off = desc[4 * img];
+  const long long off = desc[NF * img];
   // clamped so that a corrupt descriptor cannot divide by zero or overflow the index arithmetic; reads are bounded below
-  const int h = (int)min(max(desc[4 * img + 1], 1LL), 1LL << 30);
-  const int w = (int)min(max(desc[4 * img + 2], 1LL), 1LL << 30);
-  const int rw = (int)min(max(desc[4 * img + 3], 0LL), (long long)a.out_w);
+  const int h = (int)min(max(desc[NF * img + 1], 1LL), 1LL << 30);
+  const int w = (int)min(max(desc[NF * img + 2], 1LL), 1LL << 30);
+  const int rw = (int)min(max(desc[NF * img + 3], 0LL), (long long)a.out_w);
+  // the frame that is resampled (sh x sw) and its tap addresses relative to the image: base + i * si + j * sj pixels
+  int sh = h, sw = w;
+  long long si = w, sj = 1, base = 0;
+  if constexpr (ROTATED) {
+    const int k = (int)(desc[NF * img + 4] & 3);
+    if (k & 1) { sh = w; sw = h; }
+    si = k == 0 ? (long long)w : k == 1 ? -1LL : k == 2 ? -(long long)w : 1LL;
+    sj = k == 0 ? 1LL : k == 1 ? (long long)w : k == 2 ? -1LL : -(long long)w;
+    base = k == 0 ? 0LL : k == 1 ? (long long)w - 1 : k == 2 ? (long long)h * w - 1 : (long long)(h - 1) * w;
+  }
   // vertical: rows and weights of this output row
   float fly = 0.f;
-  const float fy = rw > 0 ? op_src_coord(y, h, a.out_h, &fly) : 0.f;
+  const float fy = rw > 0 ? op_src_coord(y, sh, a.out_h, &fly) : 0.f;
   const int y0 = (int)fly;
-  const long long row0 = off + 3LL * w * min(max(y0, 0), h - 1);
-  const long long row1 = off + 3LL * w * min(max(y0 + 1, 0), h - 1);
+  long long row0, row1;
+  if constexpr (ROTATED) {
+    row0 = off + 3LL * (base + si * min(max(y0, 0), sh - 1));
+    row1 = off + 3LL * (base + si * min(max(y0 + 1, 0), sh - 1));
+  } else {
+    row0 = off + 3LL * w * min(max(y0, 0), h - 1);
+    row1 = off + 3LL * w * min(max(y0 + 1, 0), h - 1);
+  }
   const int b0 = op_coef(__fsub_rn(1.f, fy)), b1 = op_coef(fy);
   const size_t plane = (size_t)a.out_h * a.out_w;
   float* o = out + (size_t)img * 3 * plane + (size_t)y * a.out_w;
@@ -59,13 +85,13 @@ __global__ void __launch_bounds__(OP_THREADS) ocr_prep_kernel(const uint8_t* __r
     int u[3] = {a.pad, a.pad, a.pad};
     if (x < rw) {
       float flx;
-      float fx = op_src_coord(x, w, rw, &flx);
+      float fx = op_src_coord(x, sw, rw, &flx);
       int x0;
       if (flx < 0.f) { x0 = 0; fx = 0.f; }
-      else if (flx >= (float)(w - 1)) { x0 = w - 1; fx = 0.f; }
+      else if (flx >= (float)(sw - 1)) { x0 = sw - 1; fx = 0.f; }
       else x0 = (int)flx;
       const int a0 = op_coef(__fsub_rn(1.f, fx)), a1 = op_coef(fx);
-      const long long c0 = 3LL * x0, c1 = 3LL * min(x0 + 1, w - 1);
+      const long long c0 = 3LL * sj * x0, c1 = 3LL * sj * min(x0 + 1, sw - 1);
       const long long at[4] = {row0 + c0, row0 + c1, row1 + c0, row1 + c1};
       int s[4][3];
 #pragma unroll
@@ -100,7 +126,8 @@ extern "C" int tpspp_ocr_prep(const tpspp_ocr_prep_cfg* cfg, const uint8_t* pack
   for (int c = 0; c < 3; ++c)
     TPSPP_REQUIRE(cfg->std[c] != 0.f, "ocr_prep: std[%d] is 0 (NormalizeOCR divides by it)", c);
   TPSPP_REQUIRE(cfg->pad_value >= 0 && cfg->pad_value <= 255, "ocr_prep: pad_value must be in [0, 255], got %d", cfg->pad_value);
-  TPSPP_REQUIRE(cfg->flags == 0, "ocr_prep: flags must be 0, got %d", cfg->flags);
+  TPSPP_REQUIRE((cfg->flags & ~TPSPP_OCR_FLAG_ROTATED) == 0, "ocr_prep: flags must be 0 or TPSPP_OCR_FLAG_ROTATED (%d), got %d",
+                TPSPP_OCR_FLAG_ROTATED, cfg->flags);
   TPSPP_REQUIRE(cfg->packed_bytes >= 0, "ocr_prep: packed_bytes must be >= 0");
   TPSPP_REQUIRE(packed && desc && out, "tpspp_ocr_prep: null pointer");
   OcrPrepArgs a;
@@ -109,8 +136,11 @@ extern "C" int tpspp_ocr_prep(const tpspp_ocr_prep_cfg* cfg, const uint8_t* pack
   for (int c = 0; c < 3; ++c) { a.mean[c] = cfg->mean[c]; a.std_[c] = cfg->std[c]; }
   a.pad = cfg->pad_value;
   a.packed_bytes = cfg->packed_bytes;
-  ocr_prep_kernel<<<dim3(cfg->n, cfg->out_h), OP_THREADS, 0, (cudaStream_t)stream>>>(
-      packed, reinterpret_cast<const long long*>(desc), out, a);
+  const long long* d = reinterpret_cast<const long long*>(desc);
+  if (cfg->flags & TPSPP_OCR_FLAG_ROTATED)
+    ocr_prep_kernel<true><<<dim3(cfg->n, cfg->out_h), OP_THREADS, 0, (cudaStream_t)stream>>>(packed, d, out, a);
+  else
+    ocr_prep_kernel<false><<<dim3(cfg->n, cfg->out_h), OP_THREADS, 0, (cudaStream_t)stream>>>(packed, d, out, a);
   count_launch();
   TPSPP_CHECK_CUDA(cudaGetLastError());
   return TPSPP_OK;

@@ -671,15 +671,19 @@ def attn_encode(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, s
 def check_ocr_desc(desc, packed_bytes: int, out_w: int) -> np.ndarray:
     """Host-side check of the ``tpspp_ocr_prep`` descriptors (the kernel reads them on the device and cannot check them without
     a host sync): ``desc`` [n, 4] int64 rows (byte offset, h, w, resize_w) of images in a packed uint8 buffer of
-    ``packed_bytes`` bytes.  Raises ``ValueError``; returns the rows as an int64 numpy array."""
+    ``packed_bytes`` bytes, or [n, 5] rows with a fifth field ``k`` in [0, 3], the quarter turns of ``np.rot90(img, k)``
+    (``h``, ``w`` are the stored image's).  Raises ``ValueError``; returns the rows as an int64 numpy array."""
     d = desc.numpy() if isinstance(desc, torch.Tensor) else np.asarray(desc)
     if isinstance(desc, torch.Tensor) and desc.device.type != "cpu":
         raise ValueError("tps_pp_b200: ocr_prep descriptors are checked on the host: pass them as a CPU tensor or numpy array")
-    if d.dtype != np.int64 or d.ndim != 2 or d.shape[1] != 4 or d.shape[0] < 1:
-        raise ValueError(f"tps_pp_b200: ocr_prep descriptors must be a non-empty int64 [n, 4] array, got {d.dtype} {d.shape}")
+    if d.dtype != np.int64 or d.ndim != 2 or d.shape[1] not in (4, 5) or d.shape[0] < 1:
+        raise ValueError(f"tps_pp_b200: ocr_prep descriptors must be a non-empty int64 [n, 4] or [n, 5] array, got {d.dtype} {d.shape}")
     off, h, w, rw = d[:, 0], d[:, 1], d[:, 2], d[:, 3]
-    for what, bad in (("h >= 1", h < 1), ("w >= 1", w < 1), ("offset >= 0", off < 0),
-                      (f"1 <= resize_w <= out_w = {out_w}", (rw < 1) | (rw > out_w))):
+    checks = [("h >= 1", h < 1), ("w >= 1", w < 1), ("offset >= 0", off < 0),
+              (f"1 <= resize_w <= out_w = {out_w}", (rw < 1) | (rw > out_w))]
+    if d.shape[1] == 5:
+        checks.append(("0 <= k <= 3 (quarter turns)", (d[:, 4] < 0) | (d[:, 4] > 3)))
+    for what, bad in checks:
         if bad.any():
             i = int(np.flatnonzero(bad)[0])
             raise ValueError(f"tps_pp_b200: ocr_prep descriptor {i} {d[i].tolist()} breaks {what}")
@@ -696,6 +700,8 @@ def ocr_prep(packed: torch.Tensor, desc, out_h: int, out_w: int, mean, std, pad_
     """mmocr's ResizeOCR + ToTensorOCR + NormalizeOCR for a ragged batch in one launch (``tpspp_ocr_prep``): ``packed`` uint8
     HWC 3-channel images one after the other (1-D CUDA tensor), ``desc`` their [n, 4] int64 descriptors (byte offset, h, w,
     resize_w) ON THE HOST, checked by :func:`check_ocr_desc` before anything is launched -> [n, 3, out_h, out_w] fp32.
+    [n, 5] descriptors add ``k``: row i is then the image ``np.rot90(img, k)`` resized to (resize_w, out_h) (mmocr's
+    ``MultiRotateAugOCR``; rows may share an offset), and the call sets ``TPSPP_OCR_FLAG_ROTATED``.
     ``desc_dev``: the same descriptors already on the device (a caller that uploads them with its images in one copy);
     otherwise they are copied here.  ``out`` (optional) must be a contiguous fp32 tensor of that shape on the same device."""
     d = check_ocr_desc(desc, packed.numel(), out_w)
@@ -704,19 +710,20 @@ def ocr_prep(packed: torch.Tensor, desc, out_h: int, out_w: int, mean, std, pad_
     _require_cuda("packed", packed, torch.uint8)
     if packed.dim() != 1 or not packed.is_contiguous():
         raise RuntimeError("tps_pp_b200: ocr_prep `packed` must be a contiguous 1-D uint8 tensor")
-    n = d.shape[0]
+    n, fields = d.shape
     if desc_dev is None:
         desc_dev = torch.from_numpy(d).to(packed.device)
-    elif (desc_dev.dtype != torch.int64 or desc_dev.device != packed.device or tuple(desc_dev.shape) != (n, 4)
+    elif (desc_dev.dtype != torch.int64 or desc_dev.device != packed.device or tuple(desc_dev.shape) != (n, fields)
           or not desc_dev.is_contiguous()):
-        raise RuntimeError(f"tps_pp_b200: ocr_prep `desc_dev` must be a contiguous int64 [{n}, 4] tensor on {packed.device}")
+        raise RuntimeError(f"tps_pp_b200: ocr_prep `desc_dev` must be a contiguous int64 [{n}, {fields}] tensor on {packed.device}")
     shape = (n, 3, int(out_h), int(out_w))
     if out is None:
         out = torch.empty(tuple(max(s, 0) for s in shape), dtype=torch.float32, device=packed.device)
     elif out.dtype != torch.float32 or out.device != packed.device or tuple(out.shape) != shape or not out.is_contiguous():
         raise RuntimeError(f"tps_pp_b200: ocr_prep `out` must be a contiguous fp32 {list(shape)} tensor on {packed.device}")
+    flags = N.OCR_FLAG_ROTATED if fields == 5 else 0
     cfg = N.OcrPrepCfg(n, int(out_h), int(out_w), (ctypes.c_float * 3)(*[float(m) for m in mean]),
-                       (ctypes.c_float * 3)(*[float(s) for s in std]), int(pad_value), 0, packed.numel())
+                       (ctypes.c_float * 3)(*[float(s) for s in std]), int(pad_value), flags, packed.numel())
     with torch.cuda.device(packed.device):
         N.check(N.lib().tpspp_ocr_prep(ctypes.byref(cfg), _ptr(packed), _ptr(desc_dev), _ptr(out), _stream(packed)), "tpspp_ocr_prep")
     return out

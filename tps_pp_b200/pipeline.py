@@ -13,7 +13,15 @@ formatting transforms) is a list of per-image host transforms::
 reference's kwargs and the per-image host arithmetic (ResizeOCR's width rule); the pixel work -- resize, ``/255``,
 mean/std normalisation and padding for the whole batch -- is one ``tpspp_ocr_prep`` launch over the packed uint8 images
 (``functional.ocr_prep``), writing the [N, 3, height, max_width] fp32 tensor the recogniser reads.  Only that sequence
-(Load, ResizeOCR, ToTensorOCR, NormalizeOCR, Collect) with the cv2 backend and a fixed ``max_width`` is supported.
+(Load, ResizeOCR, ToTensorOCR, NormalizeOCR, Collect) with the cv2 backend and a fixed ``max_width`` is supported, or the
+rotation test-time augmentation of mmocr's attention recognisers around the last four::
+
+    [dict(type='LoadImageFromFile'),
+     dict(type='MultiRotateAugOCR', rotate_degrees=[0, 90, 270],
+          transforms=[dict(type='ResizeOCR', ...), dict(type='ToTensorOCR'), dict(type='NormalizeOCR', ...),
+                      dict(type='Collect', ...)])]
+
+where each rotation of an image is one more descriptor over the same packed bytes, resampled rotated by the same launch.
 """
 from __future__ import annotations
 
@@ -136,7 +144,7 @@ class NormalizeOCR:
         self.mean, self.std = mean, std
 
 
-META_KEYS = ("filename", "ori_shape", "img_shape", "resize_shape", "pad_shape", "valid_ratio")
+META_KEYS = ("filename", "ori_filename", "ori_shape", "img_shape", "resize_shape", "pad_shape", "valid_ratio", "img_norm_cfg")
 
 
 @PIPELINES.register_module()
@@ -165,18 +173,87 @@ def _build(t):
     return t
 
 
+class MultiRotateAugOCR:
+    """mmocr 0.4 ``MultiRotateAugOCR`` (datasets/pipelines/test_time_aug.py): each image taller than it is wide (every image
+    with ``force_rotate``) is read once per degree of ``rotate_degrees``, rotated counter-clockwise (``np.rot90(img, d //
+    90)``); any other image once, unrotated.  ``rotate_degrees``: an int or a list of ints in [0, 360), multiples of 90; 0 is
+    appended when missing; ``None`` is ``[0]``.  ``transforms`` must be ResizeOCR, ToTensorOCR, NormalizeOCR, Collect.
+
+    It is not registered in ``PIPELINES``: :class:`TestPipeline` takes it, as a config dict or an instance, as the transform
+    after the loader and runs the rotations inside its one ``tpspp_ocr_prep`` launch."""
+
+    def __init__(self, transforms, rotate_degrees=None, force_rotate=False):
+        if not isinstance(transforms, (list, tuple)) or len(transforms) == 0:
+            raise ValueError(f"tps_pp_b200.MultiRotateAugOCR: transforms must be a non-empty list, got {transforms!r}")
+        ts = []
+        for i, t in enumerate(transforms):
+            try:
+                ts.append(_build(t))
+            except (TypeError, ValueError) as e:
+                raise ValueError(f"tps_pp_b200.MultiRotateAugOCR: transforms[{i}]: {e}") from e
+        if len(ts) != len(_ORDER) - 1 or not all(isinstance(t, kinds) for t, kinds in zip(ts, _ORDER[1:])):
+            raise ValueError(f"tps_pp_b200.MultiRotateAugOCR: transforms must be ResizeOCR, ToTensorOCR, NormalizeOCR, Collect; got "
+                             f"{[type(t).__name__ for t in ts]}")
+        if rotate_degrees is None:
+            degrees = [0]
+        else:
+            degrees = list(rotate_degrees) if isinstance(rotate_degrees, list) else [rotate_degrees]
+            for d in degrees:
+                if isinstance(d, bool) or not isinstance(d, int) or not 0 <= d < 360 or d % 90 != 0:
+                    raise ValueError(f"tps_pp_b200.MultiRotateAugOCR: rotate_degrees must be ints in [0, 360) that are multiples of "
+                                     f"90, got {rotate_degrees!r}")
+            if 0 not in degrees:
+                degrees.append(0)
+        self.transforms = ts
+        self.rotate_degrees = degrees
+        self.force_rotate = bool(force_rotate)
+        # the reference iterates set(rotate_degrees); for these values (0, 90, 180, 270) CPython's set yields them ascending
+        self._candidates = sorted(set(degrees))
+
+    def degrees(self, h: int, w: int) -> List[int]:
+        """The rotations, in degrees, that an h x w image is read in, in the reference's order."""
+        return list(self._candidates) if self.force_rotate or h > w else [0]
+
+
+def _is_rotate(t) -> bool:
+    return isinstance(t, MultiRotateAugOCR) or (isinstance(t, dict) and t.get("type") == "MultiRotateAugOCR")
+
+
+def _build_rotate(t) -> MultiRotateAugOCR:
+    if isinstance(t, MultiRotateAugOCR):
+        return t
+    kw = {k: v for k, v in t.items() if k != "type"}
+    unknown = sorted(set(kw) - {"transforms", "rotate_degrees", "force_rotate"})
+    if unknown or "transforms" not in kw:
+        raise ValueError(f"tps_pp_b200.MultiRotateAugOCR takes transforms, rotate_degrees and force_rotate; got {sorted(kw)}")
+    return MultiRotateAugOCR(**kw)
+
+
 class TestPipeline:
     """``test_pipeline`` config list -> a callable ``imgs -> (img [N, 3, height, max_width] fp32 on ``device``, img_metas)``.
 
     ``imgs`` is a non-empty list of uint8 [H, W, 3] arrays and/or image paths.  The images are packed, with their
     descriptors, into one pinned host buffer, copied to the device in one ``non_blocking`` copy, and turned into the batch
     tensor by one ``tpspp_ocr_prep`` launch on the current stream.  The pinned buffer is reused by the next call once the
-    copy that reads it has completed."""
+    copy that reads it has completed.
+
+    With :class:`MultiRotateAugOCR` (``self.rotate``) the batch holds every image's rotations, consecutively and in the
+    reference's order, ``[N', 3, height, max_width]``, and ``img_metas`` is a list of N lists: one meta per rotation, as
+    mmocr's aug test takes them.  Each image is still packed and uploaded once."""
 
     __test__ = False        # not a pytest test class despite its name
 
     def __init__(self, cfg_list: Sequence, device="cuda"):
-        ts = [_build(t) for t in cfg_list]
+        cfg_list = list(cfg_list)
+        self.rotate: Optional[MultiRotateAugOCR] = None
+        if any(_is_rotate(t) for t in cfg_list):
+            if len(cfg_list) != 2 or _is_rotate(cfg_list[0]) or not _is_rotate(cfg_list[1]):
+                raise ValueError("tps_pp_b200.TestPipeline: MultiRotateAugOCR must be the second and last transform, after "
+                                 "LoadImageFromFile / LoadImageFromNdarray, and wrap ResizeOCR, ToTensorOCR, NormalizeOCR, Collect")
+            self.rotate = _build_rotate(cfg_list[1])
+            ts = [_build(cfg_list[0])] + self.rotate.transforms
+        else:
+            ts = [_build(t) for t in cfg_list]
         if len(ts) != len(_ORDER) or not all(isinstance(t, kinds) for t, kinds in zip(ts, _ORDER)):
             names = [type(t).__name__ for t in ts]
             raise ValueError(f"tps_pp_b200.TestPipeline: the pipeline must be LoadImageFromFile / LoadImageFromNdarray, ResizeOCR, "
@@ -200,30 +277,48 @@ class TestPipeline:
             raise ValueError("tps_pp_b200.TestPipeline takes a non-empty list of images")
         for i, x in enumerate(imgs):
             check_image(x, i)
-        loaded = [self.load.load(x, i) for i, x in enumerate(imgs)]
-        n = len(loaded)
-        head = 32 * n                              # [n, 4] int64 descriptors, then the pixels
-        desc = np.empty((n, 4), dtype=np.int64)
-        metas = []
+        return self.prepare([self.load.load(x, i) for i, x in enumerate(imgs)])
+
+    def _meta(self, img, fname, rw, ratio):
+        meta = dict(filename=fname, ori_filename=fname, ori_shape=tuple(img.shape), img_shape=(self.out_h, rw, 3),
+                    resize_shape=(self.out_h, rw, 3), pad_shape=(self.out_h, self.out_w, 3), valid_ratio=ratio,
+                    img_norm_cfg=dict(mean=list(self.normalize.mean), std=list(self.normalize.std)))
+        return {k: meta[k] for k in self.collect.meta_keys}
+
+    def prepare(self, loaded: List):
+        """The batch and metas of images already loaded: a list of ``(uint8 [H, W, 3] array, filename or None)``."""
+        fields = 4 if self.rotate is None else 5
+        rows, offsets, metas = [], [], []
         off = 0
-        for i, (img, fname) in enumerate(loaded):
+        for img, fname in loaded:
             h, w = img.shape[:2]
+            # every rotation of an image takes the width rule of the stored, unrotated image: this is the reference's
+            # behaviour, since its ResizeOCR reads results['img_shape'], which MultiRotateAugOCR leaves unrotated when it
+            # replaces results['img'].  The rotated pixels are then resized to (resize_w, height).
             rw, ratio = self.resize.resize_width(h, w)
-            desc[i] = (off, h, w, rw)
+            if self.rotate is None:
+                rows.append((off, h, w, rw))
+                metas.append(self._meta(img, fname, rw, ratio))
+            else:
+                degrees = self.rotate.degrees(h, w)
+                rows += [(off, h, w, rw, d // 90) for d in degrees]
+                metas.append([self._meta(img, fname, rw, ratio) for _ in degrees])
+            offsets.append(off)
             off += h * w * 3
-            meta = dict(filename=fname, ori_shape=tuple(img.shape), img_shape=(self.out_h, rw, 3), resize_shape=(self.out_h, rw, 3),
-                        pad_shape=(self.out_h, self.out_w, 3), valid_ratio=ratio)
-            metas.append({k: meta[k] for k in self.collect.meta_keys})
+        n = len(rows)
+        desc = np.array(rows, dtype=np.int64).reshape(n, fields)
+        head = 8 * fields * n                      # [n, fields] int64 descriptors, then the pixels
         TF.check_ocr_desc(desc, off, self.out_w)
         staging = self._staging_buffer(head + off)
         host = staging.numpy()
         host[:head] = desc.view(np.uint8).reshape(-1)
-        for (img, _), (o, h, w, _) in zip(loaded, desc.tolist()):
+        for (img, _), o in zip(loaded, offsets):
+            h, w = img.shape[:2]
             host[head + o:head + o + h * w * 3].reshape(h, w, 3)[...] = img
         with torch.cuda.device(self.device):
             dev = staging[:head + off].to(self.device, non_blocking=True)
             self._copied = torch.cuda.Event()
             self._copied.record()
             out = TF.ocr_prep(dev[head:], desc, self.out_h, self.out_w, self.normalize.mean, self.normalize.std,
-                              self.resize.img_pad_value, desc_dev=dev[:head].view(torch.int64).view(n, 4))
+                              self.resize.img_pad_value, desc_dev=dev[:head].view(torch.int64).view(n, fields))
         return out, metas

@@ -5,7 +5,8 @@ dictionary and the decode of class probabilities into strings.  ``NRTR`` (regist
 recognizer/nrtr.py over ``EncodeDecodeRecognizer``, recognizer/encode_decode_recognizer.py): ``backbone`` (with ``tpsnet``
 called mid-way), ``encoder``, ``decoder`` and ``label_convertor`` built from config dicts, under the reference's sub-module
 names so that ``backbone.*`` / ``tpsnet.*`` / ``encoder.*`` / ``decoder.*`` checkpoint keys load with ``strict=True``.
-Inference: ``simple_test`` (encode_decode_recognizer.py:184-225).  Training: ``forward_train`` (encode_decode_recognizer.py:
+Inference: ``simple_test`` (encode_decode_recognizer.py:184-225), and ``aug_test`` / ``merge_aug_results`` for the
+rotation test-time augmentation.  Training: ``forward_train`` (encode_decode_recognizer.py:
 ``forward_train``) -- the labels through ``AttnConvertor.str2tensor``, the encoder and the teacher-forced decoder on native
 attention and dense kernels (``nrtr_train``), ``TFLoss`` (registry ``LOSSES``; reference losses/ce_loss.py).
 """
@@ -213,7 +214,38 @@ class NRTR(nn.Module):
         self.last_train_native = TF._Attention.calls - calls == len(self.encoder.layer_stack) + 2 * len(self.decoder.layer_stack)
         return self.loss(out_dec, targets_dict, metas)
 
+    @staticmethod
+    def merge_aug_results(aug_results):
+        """encode_decode_recognizer.py ``merge_aug_results``: the results of one image's rotations, in order (each a ``dict(text,
+        score=[...])`` or a one-element list of one, as ``simple_test`` returns it) -> ``[dict(text, score)]``, the reading
+        with the highest mean character score (``sum(score) / max(1, len(text))``; ``<UKN>`` counts 5 characters).  Only a
+        strictly higher mean replaces the best so far, so on a tie the first rotation wins; ``score`` is that float."""
+        out_text, out_score = "", -1
+        for result in aug_results:
+            r = result[0] if isinstance(result, (list, tuple)) else result
+            score = sum(r["score"]) / max(1, len(r["text"]))
+            if score > out_score:
+                out_text, out_score = r["text"], score
+        return [dict(text=out_text, score=out_score)]
+
+    def aug_test(self, imgs, img_metas, **kwargs):
+        """encode_decode_recognizer.py ``aug_test``: ``imgs`` one image's rotations, a list of [1, 3, H, W] tensors;
+        ``img_metas`` a list of ``[meta]`` lists -> ``[dict(text, score)]``.  The rotations run as one ``simple_test`` batch."""
+        results = self.simple_test(torch.cat(list(imgs)), [m[0] for m in img_metas], **kwargs)
+        return self.merge_aug_results(results)
+
     def forward(self, img, img_metas=None, return_loss=False, **kwargs):
+        """``return_loss``: :meth:`forward_train`.  Otherwise, as ``BaseRecognizer.forward_test``: a list of [1, 3, H, W]
+        tensors (one image's test-time augmentations) with a list of ``[meta]`` lists goes to :meth:`aug_test`, a tensor to
+        :meth:`simple_test`."""
         if return_loss:
             return self.forward_train(img, img_metas)
+        if isinstance(img, (list, tuple)):
+            if len(img) == 0 or any(not isinstance(t, torch.Tensor) or t.dim() != 4 or t.shape[0] != 1 for t in img):
+                raise ValueError("tps_pp_b200.NRTR: aug test takes a non-empty list of [1, 3, H, W] tensors, got "
+                                 f"{[tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__ for t in img]}")
+            if (not isinstance(img_metas, (list, tuple)) or len(img_metas) != len(img)
+                    or any(not isinstance(m, (list, tuple)) or len(m) != 1 for m in img_metas)):
+                raise ValueError(f"tps_pp_b200.NRTR: aug test takes one [meta] list per image tensor ({len(img)})")
+            return self.aug_test(img, img_metas, **kwargs)
         return self.simple_test(img, img_metas, **kwargs)
