@@ -12,16 +12,16 @@ import torch
 import torch.nn.functional as F
 
 
-def _t(state, key, dtype):
+def _t(state, key, dtype, device="cpu"):
     v = state[key]
     if isinstance(v, np.ndarray):
         v = torch.from_numpy(v)
-    return v.detach().to(dtype=dtype, device="cpu")
+    return v.detach().to(dtype=dtype, device=device)
 
 
 def _linear(state, prefix, x, dtype):
-    b = _t(state, prefix + ".bias", dtype) if (prefix + ".bias") in state else None
-    return F.linear(x, _t(state, prefix + ".weight", dtype), b)
+    b = _t(state, prefix + ".bias", dtype, x.device) if (prefix + ".bias") in state else None
+    return F.linear(x, _t(state, prefix + ".weight", dtype, x.device), b)
 
 
 def _mha(state, prefix, q, k, v, mask, n_head, dk, dtype):
@@ -37,16 +37,17 @@ def _mha(state, prefix, q, k, v, mask, n_head, dk, dtype):
     return _linear(state, prefix + ".fc", out, dtype)
 
 
-def nrtr_encoder_forward(state, feat, valid_ratios=None, n_head=8, dtype=torch.float32):
-    """feat [N, C, H, W] -> [N, H*W, C]; ``valid_ratios`` -> the key mask of ``_get_mask`` (keys t < min(T, ceil(T * r)))."""
-    feat = torch.as_tensor(feat).to(dtype)
+def nrtr_encoder_forward(state, feat, valid_ratios=None, n_head=8, dtype=torch.float32, device="cpu"):
+    """feat [N, C, H, W] -> [N, H*W, C] on ``device``; ``valid_ratios`` -> the key mask of ``_get_mask`` (keys
+    t < min(T, ceil(T * r)))."""
+    feat = torch.as_tensor(feat).to(dtype=dtype, device=device)
     n, c, h, w = feat.shape
     t = h * w
     dk = c // n_head
     x = feat.reshape(n, c, t).permute(0, 2, 1).contiguous()
     mask = None
     if valid_ratios is not None:
-        mask = torch.zeros((n, t), dtype=dtype)
+        mask = torch.zeros((n, t), dtype=dtype, device=device)
         for i, vr in enumerate(valid_ratios):
             mask[i, :min(t, math.ceil(t * vr))] = 1
     i = 0
@@ -54,10 +55,10 @@ def nrtr_encoder_forward(state, feat, valid_ratios=None, n_head=8, dtype=torch.f
         p = f"layer_stack.{i}."
 
         def ln(nm, v):
-            return F.layer_norm(v, (c,), _t(state, p + nm + ".weight", dtype), _t(state, p + nm + ".bias", dtype), 1e-5)
+            return F.layer_norm(v, (c,), _t(state, p + nm + ".weight", dtype, device), _t(state, p + nm + ".bias", dtype, device), 1e-5)
 
         hn = ln("norm1", x)
         x = x + _mha(state, p + "attn", hn, hn, hn, mask, n_head, dk, dtype)
         x = x + _linear(state, p + "mlp.w_2", F.gelu(_linear(state, p + "mlp.w_1", ln("norm2", x), dtype)), dtype)
         i += 1
-    return F.layer_norm(x, (c,), _t(state, "layer_norm.weight", dtype), _t(state, "layer_norm.bias", dtype), 1e-5)
+    return F.layer_norm(x, (c,), _t(state, "layer_norm.weight", dtype, device), _t(state, "layer_norm.bias", dtype, device), 1e-5)

@@ -78,6 +78,7 @@ def test_linear_rejects_cpu_tensors():
         TF.linear(torch.zeros(4, 8), torch.zeros(3, 8), None)
 
 
+# on 148 SMs the "unsplit" ids take split-K too; tests/test_recognizer_batch_gpu.py covers the unsplit paths at the NRTR shapes
 @pytest.mark.parametrize("rows,k,n", [(256, 512, 512), (1024, 512, 256), (256, 256, 512), (128, 64, 64)], ids=["split-K", "unsplit", "K=256", "small"])
 def test_prepared_linear_residual_gelu(rows, k, n):
     """The inference form a transformer layer needs: act(x w^T + b) + residual in the dense kernel's epilogue (or in the split-K
@@ -101,6 +102,7 @@ def test_prepared_linear_residual_gelu(rows, k, n):
         assert torch.equal(inplace, y)
 
 
+# on 148 SMs the "unsplit" ids take split-K too; tests/test_recognizer_batch_gpu.py covers the unsplit paths at the NRTR shapes
 @pytest.mark.parametrize("rows,k,n", [(256, 512, 512), (1024, 512, 256), (256, 256, 128), (64, 48, 128), (256, 512, 1024), (128, 1024, 768)],
                          ids=["split-K", "unsplit", "K=256", "cuda-core", "N=1024", "N=768"])
 def test_prepared_linear_with_layernorm_output(rows, k, n):
