@@ -239,6 +239,10 @@ __global__ void __launch_bounds__(ST_THREADS, 2) warp_fwd_staged_kernel(StagedAr
           r1[j] = blend4(r[0], r[t1[j].dx], r[t1[j].dy], r[t1[j].dy + t1[j].dx], t1[j].w);
         }
       }
+      // The stage is read through the generic proxy and refilled by the producer's bulk copy, which writes through the async
+      // proxy: without this fence the refill may land before these reads have been performed (seen as a few wrong src1 taps
+      // per B = 256 call once the grid overlaps its neighbours under programmatic dependent launch)
+      fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tail->empty[s]);   // the stage may be refilled
 #pragma unroll
